@@ -8,6 +8,7 @@ NCCL all-reduce of the float64 moment sums (advantage + observation statistics) 
 
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference ...                     # CPU oracle port on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/*.npy
 """
 import argparse
 import json
@@ -32,6 +33,7 @@ TRAFFIC_PROFILES = ("profiles/r02_play_h1_tp_raw.csv", "profiles/r01d_play_h1_tp
 N_ENVS = 4096
 HORIZON = 500
 GAMMA, LAM = 0.99, 0.97
+DUMP_BYTES = 60_000_000            # --dump-outputs: the sampled arrays; with the .npy headers well below 64 MB
 
 
 def workload_config(n, T):
@@ -256,6 +258,38 @@ def compact(d):
     return keep
 
 
+def dump_sample(out, vt, adv, mom, budget=DUMP_BYTES):
+    """What one step of the timed path hands its caller, gathered on the device: the rollout buffers ([T, C, n] or
+    [T, n]) and the value targets and normalised advantages ([T, n]) of a fixed, seeded sample of envs (``env_index``)
+    and steps (``step_index``), and copies of the float64 moment sums over all envs (``adv_moments`` [3], ``obs_moments``
+    [65]).  As many envs as fit in ``budget`` bytes keep every step; only when one env's steps alone exceed it are the
+    steps sampled as well."""
+    import torch
+    arrays = dict(out, v_target=vt, adv=adv)
+    T, n = adv.shape
+    per_cell = sum((v[0].numel() // n) * (4 if v.dtype == torch.float32 else 8) for v in arrays.values())  # one (step, env)
+    cells = max(1, (budget - 8 * (mom.numel() + n + T)) // per_cell)
+    n_env = min(n, max(1, cells // T))
+    n_t = min(T, cells // n_env)
+    rng = np.random.default_rng(0)
+    envs = np.sort(rng.choice(n, size=n_env, replace=False))
+    steps = np.arange(T) if n_t == T else np.sort(rng.choice(T, size=n_t, replace=False))
+    e_sel, t_sel = (torch.as_tensor(i, device=adv.device) for i in (envs, steps))
+    sample = {k: v.index_select(0, t_sel).index_select(v.dim() - 1, e_sel) for k, v in arrays.items()}
+    sample.update(adv_moments=mom[:3].clone(), obs_moments=mom[3:].clone(), env_index=envs, step_index=steps)
+    return sample
+
+
+def write_dump(path, sample):
+    """``dump_sample``'s arrays as ``path/<name>.npy``: float32 results stay float32, integer and flag buffers and the
+    indices are written as float64."""
+    path = Path(path)
+    path.mkdir(parents=True, exist_ok=True)
+    for k, v in sample.items():
+        v = v if isinstance(v, np.ndarray) else v.cpu().numpy()
+        np.save(path / f"{k}.npy", v if v.dtype in (np.float32, np.float64) else v.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------- our arm
 def run_ours(args):
     import torch
@@ -332,11 +366,17 @@ def run_ours(args):
     sampler.start()
     t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0.record()
-    for i in range(args.steps):
+    # only the last step's results are held: holding each step's while the next one allocates its own would make the
+    # caching allocator grow inside the timed region
+    for i in range(args.steps - 1):
         hot_step(i)
+    last_step = hot_step(args.steps - 1)
     t1.record()
     sync_all()
     launches = Kn.launch_count()
+    # gathered on the device before the end-to-end leg reuses the buffers; copied and written once the clocks are sampled
+    dump = dump_sample(*last_step, mom) if args.dump_outputs and rank == 0 else None
+    del last_step                                              # the end-to-end leg starts from the same allocator state
     ms = torch.tensor([t0.elapsed_time(t1)], device="cuda", dtype=torch.float64)
     kms = torch.tensor([sum(a.elapsed_time(b) for a, b in zip(ev_k0, ev_k1)) / args.steps], device="cuda", dtype=torch.float64)
     if world > 1:
@@ -377,7 +417,7 @@ def run_ours(args):
             vals.record_stream(copy_stream)
             copied[b] = torch.cuda.Event()
             copied[b].record(copy_stream)
-    e2e_steps = max(4, min(args.steps, 10))
+    e2e_steps = args.steps
     for i in range(2):
         e2e_step(i)
     # The end-to-end leg is bound by the HOST path (PCIe + host memory of a shared machine: profiles/r02d_probe_d2h.json),
@@ -400,6 +440,9 @@ def run_ours(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         e2e_runs.append(float(t))
     clocks = sampler.stop()                                    # sampled across the timed regions (device-resident + e2e)
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
+        del dump
     e2e_ms = min(e2e_runs)
     host = hosts[0]
     h2d = values_host.numel() * 4
@@ -518,7 +561,13 @@ def main():
     ap.add_argument("--nccl", action="store_true", help="use NCCL for the moment all-reduce instead of the NVLink mailbox kernel")
     ap.add_argument("--cpu-budget", type=float, default=15.0)
     ap.add_argument("--verbose-other", action="store_true", help="full side-measurement dictionaries on stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results (a fixed sample, at most 64 MB) as "
+                    "DIR/*.npy; --impl ours only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
     # stdout carries exactly one JSON line: whatever libraries print at the C level (NCCL's version banner under
     # NCCL_DEBUG=VERSION/WARN ...) is sent to stderr for the duration of the run
     sys.stdout.flush()

@@ -376,22 +376,63 @@ def test_a3_threshold_decisions_are_float64_exact_on_host(a3_model):
         assert np.array_equal(got_reached, cases["want_reached"]), np.flatnonzero(got_reached != cases["want_reached"])
 
 
-def test_unitree_h1_variants_from_shipped_tables():
+def _mjcf_of(m):
+    """An MJCF document that compiles to the model ``m``: its bodies with explicit inertials, joints with axis, anchor,
+    range, limited flag and reference position, sites, and one motor per actuator (slide / hinge joints only)."""
+    import xml.etree.ElementTree as ET
+    from olympics_mujoco_b200 import mjcf
+    f = lambda v: " ".join(repr(float(x)) for x in np.atleast_1d(v))
+    types = {v: k for k, v in mjcf._JNT_NAMES.items()}
+    root = ET.Element("mujoco", model=m.name)
+    ET.SubElement(root, "compiler", angle="radian")
+    ET.SubElement(root, "option", timestep=repr(m.timestep))
+    elems = {0: ET.SubElement(root, "worldbody")}
+    for b in range(m.nbody):                             # body ids are MuJoCo's depth-first order: parents come first
+        if b > 0:
+            e = elems[b] = ET.SubElement(elems[int(m.body_parentid[b])], "body", name=m.body_names[b],
+                                         pos=f(m.body_pos[b]), quat=f(m.body_quat[b]))
+            ET.SubElement(e, "inertial", pos=f(m.body_ipos[b]), mass=f(m.body_mass[b]))
+        for j in np.flatnonzero(m.jnt_bodyid == b):
+            assert int(m.jnt_type[j]) in (mjcf.JNT_SLIDE, mjcf.JNT_HINGE)
+            ET.SubElement(elems[b], "joint", name=m.jnt_names[j], type=types[int(m.jnt_type[j])], axis=f(m.jnt_axis[j]),
+                          pos=f(m.jnt_pos[j]), range=f(m.jnt_range[j]), limited=str(bool(m.jnt_limited[j])).lower(),
+                          ref=f(m.qpos0[m.jnt_qposadr[j]]))
+        for s in np.flatnonzero(m.site_bodyid == b):
+            ET.SubElement(elems[b], "site", name=m.site_names[s], pos=f(m.site_pos[s]), quat=f(m.site_quat[s]))
+    act = ET.SubElement(root, "actuator")
+    for a in range(m.nu):
+        ET.SubElement(act, "motor", name=m.actuator_names[a], joint=m.actuator_joint[a], gear=f(m.actuator_gear[a]),
+                      ctrlrange=f(m.actuator_ctrlrange[a]), ctrllimited=str(bool(m.actuator_ctrllimited[a])).lower())
+    return ET.tostring(root, encoding="unicode")
+
+
+def _assert_same_model(m, ref, what):
+    from olympics_mujoco_b200 import mjcf
+    for k in mjcf.KinematicModel._ARRAYS:
+        assert np.array_equal(np.asarray(getattr(m, k)), np.asarray(getattr(ref, k))), (what, k)
+    for k in ("jnt_names", "actuator_names", "actuator_joint", "body_names", "site_names", "nq", "nv"):
+        assert getattr(m, k) == getattr(ref, k), (what, k)
+
+
+def test_unitree_h1_variants_from_shipped_tables(tmp_path):
     """UnitreeH1.py:38-111: every constructor variant (arms, back joint, carried weight) is derived from the shipped tables
-    by table-level edits; each equals a fresh compile of the edited MJCF (when the reference is at hand) and its kinematics
-    equal the INDEPENDENT checker's fixture (always)."""
+    by table-level edits; each equals a compile of the MJCF with the constructor's edits, and its kinematics equal the
+    INDEPENDENT checker's fixture.  The shipped tables are the compiles of the reference's h1.xml (tools/gen_models.py):
+    unitree_h1_arms.json unedited, unitree_h1.json with the arms removed and re-oriented.  The MJCF compiled here is
+    written back out of unitree_h1_arms.json; it is first shown to compile to exactly that table and, with the arm edits,
+    to exactly unitree_h1.json."""
     from olympics_mujoco_b200 import mjcf
     from oracle import kinematics as K
     g = np.load(ROOT / "tests" / "golden" / "fk_independent_ref.npz")
-    xml = Path("/root/reference/olympic_mujoco/environments/data/unitree_h1/h1.xml")
+    full, default = mjcf.load_builtin("unitree_h1_arms"), mjcf.load_builtin("unitree_h1")
+    xml = tmp_path / "h1.xml"
+    xml.write_text(_mjcf_of(full))
+    _assert_same_model(mjcf.compile_unitree_h1(xml, disable_arms=False), full, "MJCF written out of unitree_h1_arms.json")
+    _assert_same_model(mjcf.compile_unitree_h1(xml), default, "arm edits in the MJCF vs the reference's compile")
+    _assert_same_model(mjcf.unitree_h1_variant(base=full), default, "arm edits on the tables vs the reference's compile")
     for kw in (dict(), dict(disable_back_joint=True), dict(disable_arms=False), dict(disable_arms=False, disable_back_joint=True),
                dict(hold_weight=True, weight_mass=5.0)):
-        m = mjcf.unitree_h1_variant(**kw)
-        if xml.exists():
-            ref = mjcf.compile_unitree_h1(xml, **kw)
-            for k in mjcf.KinematicModel._ARRAYS:
-                assert np.array_equal(np.asarray(getattr(m, k)), np.asarray(getattr(ref, k))), (kw, k)
-            assert m.jnt_names == ref.jnt_names and m.actuator_names == ref.actuator_names and m.body_names == ref.body_names
+        _assert_same_model(mjcf.unitree_h1_variant(**kw), mjcf.compile_unitree_h1(xml, **kw), kw)
     for name, m in (("h1_noback", mjcf.unitree_h1_variant(disable_back_joint=True)),
                     ("h1_carry", mjcf.unitree_h1_variant(hold_weight=True, weight_mass=5.0))):
         out = K.forward(m, g[name + "_qpos"], g[name + "_qvel"])
@@ -433,3 +474,41 @@ def test_bench_helpers_without_a_gpu():
     assert d == {"value": 2.0, "ms_per_step": 0.12346, "timing": "graph", "frac": 0.7012, "bound": "hbm", "peak": 6454.6}
     assert bench.compact([{"value": 1.0, "timing": "eager launches"}]) == [{"value": 1.0, "timing": "eager"}]
     assert bench.compact({"error": "x"}) == {"error": "x"}
+
+
+def test_bench_dump_outputs_writes_a_fixed_sample_within_64_mb(tmp_path):
+    """bench.py --dump-outputs: every returned buffer restricted to the same seeded envs and steps, float32 kept, integer
+    and flag buffers as float64, the moment sums whole; the written files stay below 64 MB at the bench's buffer shapes
+    for any horizon (envs are sampled first, steps too once one env's horizon alone is over the budget)."""
+    import torch
+    import bench
+    from olympics_mujoco_b200 import mjcf
+    m = mjcf.load_builtin("unitree_h1")
+    widths = dict(xpos=m.nbody * 3, xquat=m.nbody * 4, site_xpos=m.nsite * 3, cvel=m.nbody * 6, obs=32)   # make_rollout_buffers
+
+    def buffers(T, n, seed):
+        g = torch.Generator().manual_seed(seed)
+        big = lambda *s: torch.randn((1,) + s[1:], generator=g).expand(*s)        # full bench shapes, one step of memory
+        out = {k: big(T, c, n) for k, c in widths.items()}
+        out.update(reward=big(T, n), fallen=torch.randint(0, 2, (1, n), dtype=torch.uint8, generator=g).expand(T, n),
+                   traj_no_t=torch.randint(0, 4, (1, n), dtype=torch.int32, generator=g).expand(T, n),
+                   step_no_t=torch.arange(T, dtype=torch.int32)[:, None].expand(T, n))
+        return out, big(T, n), big(T, n), torch.randn(68, dtype=torch.float64, generator=g)
+
+    for T, n, budget in ((500, 4096, bench.DUMP_BYTES), (1000, 4096, bench.DUMP_BYTES), (200, 50, 100_000)):
+        out, vt, adv, mom = buffers(T, n, T)
+        for d in ("a", "b"):
+            bench.write_dump(tmp_path / f"{T}{d}", bench.dump_sample(out, vt, adv, mom, budget=budget))
+        files = sorted((tmp_path / f"{T}a").glob("*.npy"))
+        assert sum(p.stat().st_size for p in files) <= budget + 256 * len(files) < 64e6
+        got = {p.stem: np.load(p) for p in files}
+        assert set(got) == {*out, "v_target", "adv", "adv_moments", "obs_moments", "env_index", "step_index"}
+        envs, steps = got["env_index"].astype(np.int64), got["step_index"].astype(np.int64)
+        assert len(set(envs)) == len(envs) and envs.max() < n and len(set(steps)) == len(steps) and steps.max() < T
+        assert (len(steps) == T) == (budget > 10 ** 6), "steps are sampled only when one env's horizon is over the budget"
+        for k, v in (*out.items(), ("v_target", vt), ("adv", adv)):
+            assert got[k].dtype == (np.float32 if v.dtype == torch.float32 else np.float64), k
+            assert np.array_equal(got[k], v.numpy()[steps][..., envs]), k
+        assert np.array_equal(got["adv_moments"], mom[:3].numpy()) and np.array_equal(got["obs_moments"], mom[3:].numpy())
+        for p in files:
+            assert p.read_bytes() == (tmp_path / f"{T}b" / p.name).read_bytes(), p.name
