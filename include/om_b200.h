@@ -85,6 +85,10 @@ int om_model_create(const OmModelDesc* desc, OmModel** out);
 void om_model_destroy(OmModel* m);
 /* 1 when the model is served by a generated (topology-specialised) kernel, 0 for the table-driven one */
 int om_model_is_specialised(const OmModel* m);
+/* Which UnitreeH1 model the tables are, for the fused playback / live-step kernels (recognised by exact table match):
+ * 1 the default (arms disabled), 2 no back joint, 3 arms, 4 arms without the back joint, 5 / 6 / 7 / 8 carrying a
+ * 0.1 / 1 / 5 / 10 kg weight; 0 for any other model.  Only the default model is also `specialised`. */
+int om_model_h1_variant(const OmModel* m);
 
 /* ------------------------------------------------------------------------------------------------
  * K1: forward kinematics + COM + COM velocity = the subset of mujoco.mj_forward the path consumes
@@ -159,13 +163,16 @@ int om_traj_next(const OmTraj* t, uint64_t seed, uint32_t env_id0, int auto_rese
  * Fused playback: LocoEnvBase.play_trajectory_from_velocity (loco_env_base.py:444-560) for n envs,
  * one episode of n_steps steps per call (call once per episode).  end_episode_reset is a bit set: OM_PLAY_END_RESET
  * performs the end-of-episode reset (:555-557), OM_PLAY_START_RESET the reset() with which every call of the reference
- * begins (:481; sample = get_current_sample(), curr_qpos = sample[:len_qpos]) -- inside the same launches.  Per step: Euler step of the 17 coordinates (:515-519),
+ * begins (:481; sample = get_current_sample(), curr_qpos = sample[:len_qpos]) -- inside the same launches.  Per step: Euler step of the NQ coordinates (:515-519),
  * set_sim_state (:659-684), K1, next sample / wrap reset (:532-537), observation from the next sample
  * (:539), has_fallen (:541), TargetVelocityReward on the previous observation.
  * State in/out: traj_no, step_no, reset_count, xy_off, curr_qpos [n_obs_q][ld] (spec order, float64),
  * pending [K][ld] (the `sample` variable of the loop), prev_x_vel [ld].
  * Outputs (any may be NULL), time-major [n_steps][C][ld]: xpos, xquat, site_xpos, cvel, obs, reward,
- * fallen (uint8), traj_no_t / step_no_t (int32 state after each step). */
+ * fallen (uint8), traj_no_t / step_no_t (int32 state after each step).
+ * Any model with om_model_h1_variant() != 0; spec->n_obs_q must be its NQ (17 default and carry, 16 no back joint, 25 arms,
+ * 24 arms without the back joint), t->K = 2 NQ and obs_perm the model's own spec order.  Per-step sizes: obs [2 NQ - 2],
+ * xpos [3 nbody], xquat [4 nbody], cvel [6 nbody], site_xpos [3 nsite] (nbody 21, 22 with a carried weight; nsite 1). */
 #define OM_PLAY_END_RESET 1
 #define OM_PLAY_START_RESET 2
 typedef struct OmPlayState {
@@ -175,8 +182,9 @@ typedef struct OmPlayState {
 typedef struct OmPlayOut {
   float* xpos; float* xquat; float* site_xpos; float* cvel; float* obs; float* reward;
   uint8_t* fallen; int32_t* traj_no_t; int32_t* step_no_t;
-  double* obs_moments;   /* [65] float64 or NULL: S1 fused into the playback -- sum[32], sumsq[32] and count of the emitted
-                            observations are ADDED (om_moments layout and semantics: zero it first, all-reduce it after) */
+  double* obs_moments;   /* [2 nobs + 1] float64 or NULL (nobs = 2 NQ - 2: 65 values for the default model, 97 with arms):
+                            S1 fused into the playback -- sum[nobs], sumsq[nobs] and count of the emitted observations are
+                            ADDED (om_moments layout and semantics: zero it first, all-reduce it after) */
 } OmPlayOut;
 int om_h1_play_from_velocity(const OmModel* m, const OmH1Spec* spec, const OmTraj* t, uint64_t seed,
                              uint32_t env_id0, double dt, int n_steps, int end_episode_reset,
@@ -194,10 +202,11 @@ int om_h1_play_trajectory(const OmModel* m, const OmH1Spec* spec, const OmTraj* 
  * MuJoCo.step: reward(self._obs, action, cur_obs, absorbing), then self._obs = cur_obs).  Replaces the three launches
  * om_traj_next -> om_set_sim_state -> om_h1_step, whose sample and qpos / qvel round-tripped through HBM.
  * State in/out: traj_no, step_no [n], reset_count [n], xy_off [2][ld] float64, prev_x_vel [ld] (row x_vel_idx of the
- * previous observation in, of this step's observation out).  Outputs, single step, any may be NULL: qpos / qvel [17][ld]
- * (the MjData mirrors), xpos [63][ld], xquat [84][ld], site_xpos [3][ld], cvel [126][ld], obs [32][ld], reward [ld],
- * absorbing [ld] uint8, wrapped [ld] uint8 (1 where the trajectory wrapped and the env was reset).  Safe to capture in a
- * CUDA graph (no host synchronisation, no allocation). */
+ * previous observation in, of this step's observation out).  Outputs, single step, any may be NULL: qpos / qvel [NQ][ld]
+ * (the MjData mirrors), xpos [3 nbody][ld], xquat [4 nbody][ld], site_xpos [3 nsite][ld], cvel [6 nbody][ld],
+ * obs [2 NQ - 2][ld], reward [ld], absorbing [ld] uint8, wrapped [ld] uint8 (1 where the trajectory wrapped and the env was
+ * reset); the default model: NQ 17, nbody 21, nsite 1.  Same models and spec rules as om_h1_play_from_velocity, and
+ * x_vel_idx = NQ - 2.  Safe to capture in a CUDA graph (no host synchronisation, no allocation). */
 typedef struct OmLiveState {
   int32_t* traj_no; int32_t* step_no; uint32_t* reset_count; double* xy_off; float* prev_x_vel;
 } OmLiveState;

@@ -105,6 +105,7 @@ PROTOTYPES = {
     "om_model_create": (_I, [C.POINTER(OmModelDesc), C.POINTER(_P)]),
     "om_model_destroy": (None, [_P]),
     "om_model_is_specialised": (_I, [_P]),
+    "om_model_h1_variant": (_I, [_P]),
     "om_fk": (_I, [_P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _I, _P]),
     "om_h1_step": (_I, [_P, C.POINTER(OmH1Spec), _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "om_set_sim_state": (_I, [_P, C.POINTER(OmH1Spec), _P, _I, _I, _P, _P, _P]),

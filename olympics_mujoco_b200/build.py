@@ -18,6 +18,7 @@ from . import codegen, mjcf
 PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 GEN = CSRC / "gen"
+H1V = GEN / "h1v"
 LIB = PKG / "libom_b200.so"
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
@@ -66,6 +67,59 @@ def generate():
            "".join(f"constexpr int OM_A3_{k} = {v};\n" for k, v in ids.items()) +
            f"constexpr float OM_A3_TOTAL_MASS = {codegen._f(a3.total_mass)};\n")
     _write_if_changed(GEN / "a3_ids.h", txt)
+    _generate_h1_variants()
+
+
+# The UnitreeH1 constructor variants with fused playback / live-step kernels: (name, unitree_h1_variant kwargs).  Id 1 is the
+# default model (arms disabled, back joint kept); the ids below follow it.  A carried weight changes the FK (the COM and
+# cvel see its mass), so each valid weight is a model of its own, recognised by exact table match like the others.
+H1_VARIANTS = [("noback", dict(disable_back_joint=True)),
+               ("arms", dict(disable_arms=False)),
+               ("arms_noback", dict(disable_arms=False, disable_back_joint=True))] + \
+              [(f"carry_{str(w).rstrip('0').rstrip('.').replace('.', 'p')}", dict(hold_weight=True, weight_mass=w))
+               for w in mjcf.H1_VALID_WEIGHTS]
+
+
+def _generate_h1_variants():
+    """Per variant, into gen/h1v/ (build products, not kept in git): FK + observation permutation + kernel descriptor
+    (<name>.cuh) and the model tables it is recognised by (tables_<name>.h); list.h lists (id, name) for the model and
+    trajectory code, tables.h includes every table.  om_traj.cu is compiled once per variant against its descriptor."""
+    from .synthetic import H1_SPEC_JOINTS as ALL_SPEC_JOINTS
+    H1V.mkdir(exist_ok=True)
+    listing, tables = [], []
+    for vid, (name, kw) in enumerate(H1_VARIANTS, start=2):
+        m = mjcf.unitree_h1_variant(**kw)
+        js = [j for j in ALL_SPEC_JOINTS if j in m.jnt_names]
+        perm = [int(m.jnt_qposadr[m.jnt_names.index(j)]) for j in js]
+        assert len(perm) == m.nq == m.nv, name
+        up, p = name.upper(), ", ".join(map(str, perm))
+        txt = ("#pragma once\n" + codegen.generate_fk(m, f"om_fk_h1v_{name}") +
+               f"// GENERATED: qpos/qvel address of observation-spec entry k\n"
+               f"__device__ constexpr int OM_H1V_{up}_PERM[{m.nq}] = {{{p}}};\n"
+               f"static const int OM_H1V_{up}_PERM_HOST[{m.nq}] = {{{p}}};\n"
+               f"struct H1V_{name} {{\n"
+               f"  static constexpr int ID = {vid}, NQ = {m.nq}, NBODY = {m.nbody}, NSITE = {m.nsite};\n"
+               f"  static OM_HD int perm(int k) {{ return OM_H1V_{up}_PERM[k]; }}\n"
+               f"  static const int* perm_host() {{ return OM_H1V_{up}_PERM_HOST; }}\n"
+               f"  template <class Sink>\n"
+               f"  static OM_HD void fk(const float (&q)[NQ], const float (&qd)[NQ], Sink& S) {{ om_fk_h1v_{name}(q, qd, S); }}\n"
+               f"}};\n")
+        _write_if_changed(H1V / f"{name}.cuh", txt)
+        _write_if_changed(H1V / f"tables_{name}.h", "#pragma once\n" + codegen.generate_tables(m, f"om_tab_h1v_{name}"))
+        listing.append(f"X({vid}, {name})")
+        tables.append(f'#include "tables_{name}.h"\n')
+    _write_if_changed(H1V / "list.h",
+                      "#pragma once\n// GENERATED: (variant id, name) of every UnitreeH1 variant with its own kernels\n"
+                      "#define OM_H1_VARIANTS(X) " + " ".join(listing) + "\n")
+    _write_if_changed(H1V / "tables.h", "#pragma once\n" + "".join(tables))
+
+
+def compile_units():
+    """(source, extra nvcc flags, object name): every .cu once, and om_traj.cu once more per UnitreeH1 variant."""
+    units = [(src, [], src.stem) for src in sources()]
+    units += [(CSRC / "om_traj.cu", [f"-DOM_H1_VARIANT={name}", f'-DOM_H1_VARIANT_HEADER="gen/h1v/{name}.cuh"'],
+               f"om_traj_h1v_{name}") for name, _ in H1_VARIANTS]
+    return units
 
 
 def sources():
@@ -74,7 +128,7 @@ def sources():
 
 def _digest():
     h = hashlib.sha256()
-    for p in sorted(list(CSRC.glob("*.cu")) + list(CSRC.glob("*.cuh")) + list(GEN.glob("*")) +
+    for p in sorted(list(CSRC.glob("*.cu")) + list(CSRC.glob("*.cuh")) + list(GEN.glob("*.*")) + list(H1V.glob("*")) +
                     [PKG.parent / "include" / "om_b200.h", Path(__file__)]):
         h.update(p.name.encode())
         h.update(p.read_bytes())
@@ -91,16 +145,16 @@ def build(force=False, verbose=True):
     objdir = PKG / "build"
     objdir.mkdir(exist_ok=True)
     procs = []
-    for src in sources():
-        obj = objdir / (src.stem + ".o")
-        cmd = [NVCC, *ARCH, *FLAGS, "-I", str(PKG.parent / "include"), "-c", str(src), "-o", str(obj)]
-        procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
+    for src, extra, stem in compile_units():
+        obj = objdir / (stem + ".o")
+        cmd = [NVCC, *ARCH, *FLAGS, *extra, "-I", str(PKG.parent / "include"), "-c", str(src), "-o", str(obj)]
+        procs.append((stem, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
         objs.append(obj)
     log = []
     failed = False
-    for src, p in procs:
+    for stem, p in procs:
         out, _ = p.communicate()
-        log.append(f"==== {src.name}\n{out}")
+        log.append(f"==== {stem}\n{out}")
         if p.returncode != 0:
             failed = True
     (objdir / "ptxas.log").write_text("\n".join(log))

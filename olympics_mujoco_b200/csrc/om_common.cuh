@@ -102,6 +102,7 @@ struct OmModel {
   om::ModelTab host;
   om::ModelTab* dev = nullptr;
   int specialised = om::SPEC_NONE;
+  int h1_variant = 0;   // UnitreeH1 model with fused playback / live-step kernels: 1 default, 2.. gen/h1v/list.h; else 0
   int device = 0;
 };
 

@@ -6,6 +6,8 @@
 #include "om_common.cuh"
 #include "gen/tables_unitree_h1.h"
 #include "gen/tables_stick_figure_a3.h"
+#include "gen/h1v/list.h"
+#include "gen/h1v/tables.h"
 
 namespace om {
 
@@ -135,6 +137,12 @@ extern "C" int om_model_create(const OmModelDesc* d, OmModel** out) {
   }
   if (OM_MATCH(om_tab_h1, t)) m->specialised = SPEC_H1;
   else if (OM_MATCH(om_tab_a3, t)) m->specialised = SPEC_A3;
+  // the UnitreeH1 variants with fused playback / live-step kernels; only the default model is `specialised` (om_fk and
+  // om_h1_step keep the table-driven FK for the others)
+  if (m->specialised == SPEC_H1) m->h1_variant = 1;
+#define OM_H1_VARIANT_MATCH(id, name) else if (OM_MATCH(om_tab_h1v_##name, t)) m->h1_variant = id;
+  OM_H1_VARIANTS(OM_H1_VARIANT_MATCH)
+#undef OM_H1_VARIANT_MATCH
   cudaGetDevice(&m->device);
   cudaError_t e = cudaMalloc(&m->dev, sizeof(ModelTab));
   if (e == cudaSuccess) e = cudaMemcpy(m->dev, &t, sizeof(ModelTab), cudaMemcpyHostToDevice);
@@ -153,3 +161,4 @@ extern "C" void om_model_destroy(OmModel* m) {
 }
 
 extern "C" int om_model_is_specialised(const OmModel* m) { return m ? m->specialised : 0; }
+extern "C" int om_model_h1_variant(const OmModel* m) { return m ? m->h1_variant : 0; }

@@ -9,8 +9,9 @@ struct TrajDev {
   const double* xy;    // [n_traj][T][2]   channels 0,1 (root x, y) in float64
   const double* cdq;   // [n_traj][T+1][K/2] exclusive prefix sums of the velocity channels (float64):
                        //   cdq[tr][i][k] = sum_{j<i} rows[tr][j][K/2+k]  (time-parallel playback)
-  const double* psum;  // [n_traj][T+1][64] exclusive prefix sums of the observation rows (channels 2..33) and of their
-                       //   squares, float64 (S1 of a playback call as prefix differences); null unless K == 34
+  const double* psum;  // [n_traj][T+1][2 (K-2)] exclusive prefix sums of the observation rows (channels 2..K-1) and of
+                       //   their squares, float64 (S1 of a playback call as prefix differences); null unless K is the
+                       //   key count of a UnitreeH1 model with fused kernels (32, 34, 48 or 50)
   int K, kpad, n_traj, T;
 };
 
@@ -21,11 +22,13 @@ OM_HD void traj_draw(const TrajDev& t, uint64_t seed, uint32_t env_id, uint32_t 
   step_no = to_int(w.y, t.T);
 }
 
-// one sample row into registers (kpad <= 36 for the H1 table); vectorised 16-byte gathers
-OM_HD void traj_load_row(const TrajDev& t, int traj_no, int step_no, float (&samp)[36]) {
+// one sample row into registers (KPAD == t.kpad, checked on the host); vectorised 16-byte gathers
+template <int KPAD>
+OM_HD void traj_load_row(const TrajDev& t, int traj_no, int step_no, float (&samp)[KPAD]) {
+  static_assert(KPAD % 4 == 0, "rows are padded to whole float4s");
   const float4* r = reinterpret_cast<const float4*>(t.rows + ((size_t)traj_no * t.T + step_no) * t.kpad);
 #pragma unroll
-  for (int v = 0; v < 9; ++v) {
+  for (int v = 0; v < KPAD / 4; ++v) {
     const float4 x = __ldg(r + v);
     samp[4 * v] = x.x; samp[4 * v + 1] = x.y; samp[4 * v + 2] = x.z; samp[4 * v + 3] = x.w;
   }

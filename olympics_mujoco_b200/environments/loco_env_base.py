@@ -229,7 +229,14 @@ class LocoEnvBase:
         self._data.qvel.zero_()                                                              # mj_resetData
         if self._grf is not None:
             self._grf.zero_()                                                                # mean_grf.reset() :584
-        if len(self._models) > 1:                                                            # MultiMuJoCo :586-599
+        self._next_model()
+        self.setup(obs)
+        self._obs = self._create_observation(self.obs_helper._build_obs(self._data))
+        return self._out(self._modify_observation(self._obs))
+
+    def _next_model(self):
+        """The model switch of reset() (MultiMuJoCo :586-599); nothing with a single model.  Decided on the host."""
+        if len(self._models) > 1:
             if self._random_env_reset:
                 # np.random.randint in the reference; here the Philox contract (stream 32, counter = number of resets)
                 from ..utils.philox import STREAM_MODEL_RESET, philox_randint
@@ -239,9 +246,6 @@ class LocoEnvBase:
                 self._current_model_idx = self._current_model_idx + 1 if self._current_model_idx < len(self._models) - 1 else 0
             self._model_resets += 1
             self._select_model(self._current_model_idx)
-        self.setup(obs)
-        self._obs = self._create_observation(self.obs_helper._build_obs(self._data))
-        return self._out(self._modify_observation(self._obs))
 
     def _select_model(self, idx):
         prev = self._data

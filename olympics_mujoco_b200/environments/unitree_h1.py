@@ -1,6 +1,7 @@
 """Batched ``UnitreeH1`` environment (reference ``real_humanoid_robots/UnitreeH1.py`` and
 ``base_robot/base_humanoid_robot.py``): same constructor switches, observation/action specs, ``generate``,
-``_has_fallen`` and ``is_absorbing``; ``step`` and ``play_trajectory_from_velocity`` run the fused CUDA kernels.
+``_has_fallen`` and ``is_absorbing``; ``step`` and ``play_trajectory_from_velocity`` run the fused CUDA kernels (the
+playback and live-step kernels exist for every constructor variant built from the shipped tables).
 """
 from __future__ import annotations
 
@@ -227,11 +228,14 @@ class UnitreeH1(BaseHumanoidRobot):
         return self._out(self._modify_observation(cur_obs)), self._out(reward), self._out(absorbing), {}
 
     # ------------------------------------------------------------------ fused live step / graph
+    def _has_fused_kernels(self):
+        """Every model of this env (one per carried weight with MultiMuJoCo) has generated playback / live-step kernels."""
+        return all(dm.h1_variant for dm in self._dms)
+
     def _live_stepper(self):
-        if (not self._dm.specialised or len(self.obs_helper.observation_spec) != 34 or not self._fused_reward
-                or self._use_foot_forces):
-            raise NotImplementedError("the fused live step is generated for the default UnitreeH1 (arms disabled) with the "
-                                      "target-velocity reward")
+        if not self._has_fused_kernels() or not self._fused_reward or self._use_foot_forces:
+            raise NotImplementedError("the fused live step is generated for the UnitreeH1 models of the shipped tables with "
+                                      "the target-velocity reward")
         if getattr(self, "_live", None) is None:
             if self._obs is None:
                 self.reset()
@@ -262,7 +266,7 @@ class UnitreeH1(BaseHumanoidRobot):
         n, dev = self.n_envs, self._device
         bufs = {}
         for k in want:
-            c, dt_ = Kn.H1LiveStep.KEYS[k]
+            c, dt_ = live.keys[k]
             bufs[k] = torch.empty((n_steps, n) if c is None else (n_steps, c, n), dtype=dt_, device=dev)
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream())
@@ -301,7 +305,8 @@ class UnitreeH1(BaseHumanoidRobot):
                                                   "traj_no_t", "step_no_t")):
         m, n, dev = self._model, self.n_envs, self._device
         spec = dict(xpos=(m.nbody * 3, torch.float32), xquat=(m.nbody * 4, torch.float32),
-                    site_xpos=(m.nsite * 3, torch.float32), cvel=(m.nbody * 6, torch.float32), obs=(32, torch.float32),
+                    site_xpos=(m.nsite * 3, torch.float32), cvel=(m.nbody * 6, torch.float32),
+                    obs=(2 * self._spec.n_obs_q - 2, torch.float32),
                     reward=(None, torch.float32), fallen=(None, torch.uint8), traj_no_t=(None, torch.int32),
                     step_no_t=(None, torch.int32))
         return {k: torch.empty((n_steps, n) if spec[k][0] is None else (n_steps, spec[k][0], n), dtype=spec[k][1],
@@ -311,7 +316,12 @@ class UnitreeH1(BaseHumanoidRobot):
         """Both playback calls: every call of the reference begins with ``reset()`` (:377 / :481) and ends every episode
         with one (:432 / :555).  The first call resets through the Python API (it also allocates the carried state);
         later calls perform the same reset INSIDE the first kernel of the call.  ``continue_episode=True`` (extension)
-        skips the reset at the start and carries the state of the previous call on."""
+        skips the reset at the start and carries the state of the previous call on.
+
+        With MultiMuJoCo (a carried weight of every valid mass) each reset() performed inside a kernel switches the model on
+        the host exactly as reset() does, so each episode runs on the model the preceding reset chose.  A variant model
+        called with none of ``out`` / ``want`` / ``obs_moments`` returns what the base class returns, ``dict(obs=[n, nobs]
+        last observation, has_fallen=[n])``, from the kernel's carried sample and its per-step fallen flags."""
         assert self.trajectories is not None
         if render or record:
             raise NotImplementedError("rendering is outside the hot path; call with render=False")
@@ -321,26 +331,37 @@ class UnitreeH1(BaseHumanoidRobot):
         if self._play_state is None:
             self.reset()                                                             # :377 / :481
             sample = self.trajectories.get_current_sample().t().contiguous()         # :379 / :483
-            self._play_state = dict(curr_qpos=sample[:17].double().contiguous(), pending=sample.clone(),
+            self._play_state = dict(curr_qpos=sample[:self._spec.n_obs_q].double().contiguous(), pending=sample.clone(),
                                     prev_x_vel=self._prev_x_vel)
             start_reset = False
         res = None
-        kw = {} if want is None else dict(want=want)
+        summary = not self._dm.specialised and out is None and want is None and obs_moments is None
+        kw = dict(want=("fallen",)) if summary else ({} if want is None else dict(want=want))
+        fallen_any = torch.zeros(self.n_envs, dtype=torch.bool, device=self._device) if summary else None
         for ep in range(n_episodes):
+            if start_reset and ep == 0:
+                self._next_model()                                                   # the in-kernel reset() at :377 / :481
             res = Kn.h1_play_from_velocity(self._dm, self._spec, dev, self._play_state, n_steps_per_episode, dt=self.dt,
                                            end_episode_reset=True, out=out, forced=forced, obs_moments=obs_moments,
                                            start_reset=start_reset and ep == 0, **kw)
+            if summary:
+                fallen_any |= res["fallen"].any(dim=0).bool()
+            self._next_model()                                                       # the in-kernel reset() at :432 / :555
         # the env is left in the state of the final reset() (:432 / :555): its observation is that sample's, fetched on
         # first use (the loop's `sample` variable -- our `pending` -- stays the stale one, as in the reference)
         self.__dict__["_obs_lazy"] = lambda: self._create_observation(self.trajectories.get_current_sample())
+        if summary:
+            obs = self._play_state["pending"][2:].t().clone() if n_episodes and n_steps_per_episode else None
+            return dict(obs=None if obs is None else self._out(obs), has_fallen=self._out(fallen_any))
         return res
 
     def play_trajectory(self, n_episodes=None, n_steps_per_episode=None, render=False, record=False, recorder_params=None,
                         out=None, want=None, continue_episode=False, obs_moments=None):
         """loco_env_base.py:338-442 as one fused kernel per episode (``om_h1_play_trajectory``): the model is forced to
         every trajectory sample, FK runs on it, the next sample gives the observation and the has_fallen flag.
-        Returns the last episode's time-major rollout buffers (the reference only renders)."""
-        if not self._dm.specialised or len(self.obs_helper.observation_spec) != 34:
+        Returns the last episode's time-major rollout buffers (the reference only renders); see ``_play`` for the other
+        variants' return value."""
+        if not self._has_fused_kernels() or (self._use_foot_forces and not self._dm.specialised):
             return super().play_trajectory(n_episodes, n_steps_per_episode, render, record, recorder_params)
         return self._play(True, n_episodes, n_steps_per_episode, render, record, out, want, continue_episode, obs_moments)
 
@@ -350,8 +371,9 @@ class UnitreeH1(BaseHumanoidRobot):
         start of EVERY call and after every episode -- one fused kernel per episode).  Returns the last episode's
         time-major rollout buffers ([T, C, n] SoA; use ``kernels.env_major`` for [T, n, ...] views) -- the reference
         returns nothing and only renders.  ``obs_moments``: float64 [65] buffer that receives the moment sums of the
-        emitted observations (S1 fused into the kernel)."""
-        if not self._dm.specialised or len(self.obs_helper.observation_spec) != 34 or self._use_foot_forces:
-            # other variants (arms, no back joint, carried weight, foot forces): per-step kernels of the base class
+        emitted observations (S1 fused into the kernel); ``2 nobs + 1`` values for a model with nobs observations.  See
+        ``_play`` for the return value of the other variants."""
+        if not self._has_fused_kernels() or self._use_foot_forces:
+            # a model without generated kernels (user XML, an unlisted weight) or foot forces: per-step kernels of the base class
             return super().play_trajectory_from_velocity(n_episodes, n_steps_per_episode, render, record, recorder_params)
         return self._play(False, n_episodes, n_steps_per_episode, render, record, out, want, continue_episode, obs_moments)

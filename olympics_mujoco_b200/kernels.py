@@ -78,6 +78,8 @@ class DeviceModel:
         check(lib.om_model_create(C.byref(desc), C.byref(h)))
         self.handle = h
         self.specialised = bool(lib.om_model_is_specialised(h))
+        # UnitreeH1 model with fused playback / live-step kernels: 1 the default, 2.. its other variants, 0 none
+        self.h1_variant = int(lib.om_model_h1_variant(h))
 
     def __del__(self):
         try:
@@ -207,17 +209,20 @@ class DeviceTrajectory:
 def h1_play_from_velocity(dm, spec, traj: DeviceTrajectory, state, n_steps, dt=0.01, end_episode_reset=True,
                           want=("xpos", "xquat", "site_xpos", "cvel", "obs", "reward", "fallen", "traj_no_t", "step_no_t"),
                           out=None, forced=False, obs_moments=None, start_reset=False):
-    """Fused playback of one episode (loco_env_base.py:511-557).  ``state``: dict with curr_qpos [17,n] f64,
-    pending [34,n] f32, prev_x_vel [n] f32 (the trajectory indices live in ``traj``).  ``forced``: play_trajectory
-    semantics (loco_env_base.py:404-432), the model is set to each sample instead of integrating velocities.
-    ``obs_moments``: float64 [65] device buffer; the kernel ADDS sum[32], sumsq[32], count of the observations it emits
+    """Fused playback of one episode (loco_env_base.py:511-557) on any UnitreeH1 model with ``dm.h1_variant != 0``.
+    ``state``: dict with curr_qpos [NQ,n] f64, pending [2 NQ,n] f32, prev_x_vel [n] f32 (the trajectory indices live in
+    ``traj``; NQ = ``spec.n_obs_q``, 17 for the default model).  ``forced``: play_trajectory semantics
+    (loco_env_base.py:404-432), the model is set to each sample instead of integrating velocities.
+    ``obs_moments``: float64 [2 nobs + 1] device buffer (nobs = 2 NQ - 2; 65 values for the default model); the kernel
+    ADDS sum[nobs], sumsq[nobs], count of the observations it emits
     (S1 fused into the playback: no second pass over the observation buffer).  ``start_reset``: the call begins with
     the reference's ``reset()`` (loco_env_base.py:481), performed inside the kernel (no state tensor is read before it)."""
     km, n = dm.km, traj.n
     dev = traj.traj_no.device
+    nobs = 2 * spec.n_obs_q - 2
     sizes = dict(xpos=(km.nbody * 3, torch.float32), xquat=(km.nbody * 4, torch.float32),
                  site_xpos=(km.nsite * 3, torch.float32), cvel=(km.nbody * 6, torch.float32),
-                 obs=(32, torch.float32), reward=(None, torch.float32), fallen=(None, torch.uint8),
+                 obs=(nobs, torch.float32), reward=(None, torch.float32), fallen=(None, torch.uint8),
                  traj_no_t=(None, torch.int32), step_no_t=(None, torch.int32))
     out = dict(out or {})
     for k in want:
@@ -232,8 +237,8 @@ def h1_play_from_velocity(dm, spec, traj: DeviceTrajectory, state, n_steps, dt=0
                      prev_x_vel=_p(state["prev_x_vel"], torch.float32).value)
     po = OmPlayOut(**{k: (out[k].data_ptr() if k in out else None) for k in sizes})
     if obs_moments is not None:
-        if obs_moments.numel() != 65:
-            raise ValueError("obs_moments must hold 2 * 32 + 1 float64 values")
+        if obs_moments.numel() != 2 * nobs + 1:
+            raise ValueError(f"obs_moments must hold 2 * {nobs} + 1 float64 values")
         po.obs_moments = _p(obs_moments, torch.float64).value
     flags = (1 if end_episode_reset else 0) | (2 if start_reset else 0)
     if forced:
@@ -250,21 +255,31 @@ class H1LiveStep:
     set_sim_state + FK + observation + has_fallen + reward), one ctypes call per step with no per-call marshalling --
     the eager Python loop stays within a few microseconds of host time per step.  ``out``: dict of SoA tensors (any of
     qpos, qvel, xpos, xquat, site_xpos, cvel, obs, reward, absorbing, wrapped); missing FK / mirror outputs are not
-    computed.  ``prev_x_vel`` [n] float32 is carried in place.  Graph-capturable."""
+    computed.  ``prev_x_vel`` [n] float32 is carried in place.  Graph-capturable.  ``keys``: (components, dtype) of
+    each output for this model (``KEYS``: the default model's)."""
 
     KEYS = dict(qpos=(17, torch.float32), qvel=(17, torch.float32), xpos=(63, torch.float32), xquat=(84, torch.float32),
                 site_xpos=(3, torch.float32), cvel=(126, torch.float32), obs=(32, torch.float32), reward=(None, torch.float32),
                 absorbing=(None, torch.uint8), wrapped=(None, torch.uint8))
 
+    @staticmethod
+    def keys_for(dm, spec):
+        km = dm.km
+        return dict(H1LiveStep.KEYS, qpos=(km.nq, torch.float32), qvel=(km.nv, torch.float32),
+                    xpos=(km.nbody * 3, torch.float32), xquat=(km.nbody * 4, torch.float32),
+                    site_xpos=(km.nsite * 3, torch.float32), cvel=(km.nbody * 6, torch.float32),
+                    obs=(2 * spec.n_obs_q - 2, torch.float32))
+
     def __init__(self, dm, spec, traj: DeviceTrajectory, prev_x_vel, out=None,
                  want=("xpos", "xquat", "site_xpos", "cvel", "obs", "reward", "absorbing")):
         n, dev = traj.n, traj.traj_no.device
         self.dm, self.spec, self.traj, self.n = dm, spec, traj, n
+        self.keys = self.keys_for(dm, spec)
         self.prev_x_vel = prev_x_vel
         self.out = dict(out or {})
         for k in want:
             if k not in self.out:
-                c, dt_ = self.KEYS[k]
+                c, dt_ = self.keys[k]
                 self.out[k] = torch.empty((n,) if c is None else (c, n), dtype=dt_, device=dev)
         self._fn = _lib.load().om_h1_live_step
         self.rebind()
@@ -277,7 +292,7 @@ class H1LiveStep:
         self._state = OmLiveState(traj_no=traj.traj_no.data_ptr(), step_no=traj.step_no.data_ptr(),
                                   reset_count=traj.reset_count.data_ptr(), xy_off=traj.xy_off.data_ptr(),
                                   prev_x_vel=_p(self.prev_x_vel, torch.float32).value)
-        self._out = OmLiveOut(**{k: _p(v, self.KEYS[k][1]).value for k, v in self.out.items()})
+        self._out = OmLiveOut(**{k: _p(v, self.keys[k][1]).value for k, v in self.out.items()})
         st = torch.cuda.current_stream().cuda_stream if stream is None else stream
         self._args = (self.dm.handle, C.byref(self.spec), traj.handle, traj.seed, traj.env_id0, C.byref(self._state),
                       C.byref(self._out), self.n, max(self.n, 1), C.c_void_p(st))
