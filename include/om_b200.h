@@ -89,6 +89,13 @@ int om_model_is_specialised(const OmModel* m);
  * 1 the default (arms disabled), 2 no back joint, 3 arms, 4 arms without the back joint, 5 / 6 / 7 / 8 carrying a
  * 0.1 / 1 / 5 / 10 kg weight; 0 for any other model.  Only the default model is also `specialised`. */
 int om_model_h1_variant(const OmModel* m);
+/* Per-env mass of one body: afterwards om_fk, om_h1_step, om_h1_play_from_velocity, om_h1_play_trajectory and
+ * om_h1_live_step on this model read body `body`'s mass of env i from mass[i] (DEVICE, [ld] float32, n <= ld at every
+ * call) instead of the tables.  Accepted for the UnitreeH1 carry models (om_model_h1_variant 5-8) and their "weight" body
+ * (the only body whose mass differs between them), for which it selects kernels with that mass as a runtime argument; any
+ * other model or body is an error.  The binding lasts for the model's life (the pointer is read at every call, so a CUDA
+ * graph captured afterwards stays valid); rebinding to another buffer is an error. */
+int om_model_bind_env_body_mass(OmModel* m, int body, const float* mass, int ld);
 
 /* ------------------------------------------------------------------------------------------------
  * K1: forward kinematics + COM + COM velocity = the subset of mujoco.mj_forward the path consumes
@@ -216,6 +223,16 @@ typedef struct OmLiveOut {
 } OmLiveOut;
 int om_h1_live_step(const OmModel* m, const OmH1Spec* spec, const OmTraj* t, uint64_t seed, uint32_t env_id0,
                     const OmLiveState* state, const OmLiveOut* out, int n, int ld, void* stream);
+
+/* The model switch of a MultiMuJoCo reset() (loco_env_base.py:586-599) drawn per env, for n envs whose global ids start
+ * at env_id0; count = the env object's number of model resets before this one.  Env i takes model
+ *   random != 0:  Philox(key seed; counter env_id0 + i, count, 32, 0) word 0, times n_models, high 32 bits
+ *                 (the om_traj_reset contract on stream 32 = utils/philox.py philox_randint)
+ *   random == 0:  (env_id0 + i + count + 1) mod n_models  (round robin from model 0)
+ * idx [n] int32 <- the model index, mass [n] float32 <- body_mass_host[idx] (HOST, [n_models] <= 16).  Feeds the buffer
+ * bound with om_model_bind_env_body_mass; a plain stream-ordered launch. */
+int om_h1_draw_models(uint64_t seed, uint32_t env_id0, uint32_t count, int n_models, int random,
+                      const double* body_mass_host, int32_t* idx, float* mass, int n, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K2 (A3 flavour): the tail of StickFigureA3.step (real_humanoid_robots/StickFigureA3.py:187-202) after

@@ -106,6 +106,7 @@ PROTOTYPES = {
     "om_model_destroy": (None, [_P]),
     "om_model_is_specialised": (_I, [_P]),
     "om_model_h1_variant": (_I, [_P]),
+    "om_model_bind_env_body_mass": (_I, [_P, _I, _P, _I]),
     "om_fk": (_I, [_P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _I, _P]),
     "om_h1_step": (_I, [_P, C.POINTER(OmH1Spec), _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "om_set_sim_state": (_I, [_P, C.POINTER(OmH1Spec), _P, _I, _I, _P, _P, _P]),
@@ -118,6 +119,7 @@ PROTOTYPES = {
     "om_h1_play_from_velocity": (_I, [_P, C.POINTER(OmH1Spec), _P, _U64, _U32, _D, _I, _I,
                                       C.POINTER(OmPlayState), C.POINTER(OmPlayOut), _I, _I, _P]),
     "om_h1_live_step": (_I, [_P, C.POINTER(OmH1Spec), _P, _U64, _U32, C.POINTER(OmLiveState), C.POINTER(OmLiveOut), _I, _I, _P]),
+    "om_h1_draw_models": (_I, [_U64, _U32, _U32, _I, _I, _P, _P, _P, _I, _P]),
     "om_a3_task_create": (_I, [C.POINTER(OmA3TaskDesc), C.POINTER(_P)]),
     "om_a3_task_destroy": (None, [_P]),
     "om_a3_task_step": (_I, [_P, _P, _P, _P, _P, _I, C.POINTER(OmA3State), C.POINTER(OmA3Out), _I, _I, _P]),

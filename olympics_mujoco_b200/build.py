@@ -78,47 +78,69 @@ H1_VARIANTS = [("noback", dict(disable_back_joint=True)),
                ("arms_noback", dict(disable_arms=False, disable_back_joint=True))] + \
               [(f"carry_{str(w).rstrip('0').rstrip('.').replace('.', 'p')}", dict(hold_weight=True, weight_mass=w))
                for w in mjcf.H1_VALID_WEIGHTS]
+# One more kernel set for the carry models: the mass of the jointless "weight" body is read per env at run time
+# (om_model_bind_env_body_mass), so a batch can hold every valid weight at once.  It is not a model of its own: a bound
+# carry model launches it instead of its own variant's kernels.
+H1_CARRY_ENV = "carry_env"
+
+
+def _h1_descriptor(m, name, vid, env_mass_body=None):
+    """FK + observation permutation + kernel descriptor of one variant (gen/h1v/<name>.cuh)."""
+    from .synthetic import H1_SPEC_JOINTS as ALL_SPEC_JOINTS
+    js = [j for j in ALL_SPEC_JOINTS if j in m.jnt_names]
+    perm = [int(m.jnt_qposadr[m.jnt_names.index(j)]) for j in js]
+    assert len(perm) == m.nq == m.nv, name
+    up, p = name.upper(), ", ".join(map(str, perm))
+    env = env_mass_body is not None
+    return ("#pragma once\n" + codegen.generate_fk(m, f"om_fk_h1v_{name}", env_mass_body=env_mass_body) +
+            f"// GENERATED: qpos/qvel address of observation-spec entry k\n"
+            f"__device__ constexpr int OM_H1V_{up}_PERM[{m.nq}] = {{{p}}};\n"
+            f"static const int OM_H1V_{up}_PERM_HOST[{m.nq}] = {{{p}}};\n"
+            f"struct H1V_{name} {{\n"
+            f"  static constexpr int ID = {vid}, NQ = {m.nq}, NBODY = {m.nbody}, NSITE = {m.nsite};\n"
+            f"  static constexpr bool ENV_MASS = {'true' if env else 'false'};   // fk takes the env's body mass\n"
+            f"  static OM_HD int perm(int k) {{ return OM_H1V_{up}_PERM[k]; }}\n"
+            f"  static const int* perm_host() {{ return OM_H1V_{up}_PERM_HOST; }}\n"
+            f"  template <class Sink>\n" +
+            (f"  static OM_HD void fk(const float (&q)[NQ], const float (&qd)[NQ], Sink& S, float m) "
+             f"{{ om_fk_h1v_{name}(q, qd, S, m); }}\n" if env else
+             f"  static OM_HD void fk(const float (&q)[NQ], const float (&qd)[NQ], Sink& S) {{ om_fk_h1v_{name}(q, qd, S); }}\n") +
+            f"}};\n")
 
 
 def _generate_h1_variants():
     """Per variant, into gen/h1v/ (build products, not kept in git): FK + observation permutation + kernel descriptor
     (<name>.cuh) and the model tables it is recognised by (tables_<name>.h); list.h lists (id, name) for the model and
-    trajectory code, tables.h includes every table.  om_traj.cu is compiled once per variant against its descriptor."""
-    from .synthetic import H1_SPEC_JOINTS as ALL_SPEC_JOINTS
+    trajectory code, tables.h includes every table.  om_traj.cu is compiled once per variant against its descriptor.
+    carry_env.cuh: the carry model with the weight's mass as a runtime argument (no tables: no model is recognised as it)."""
     H1V.mkdir(exist_ok=True)
-    listing, tables = [], []
+    listing, tables, carry_ids = [], [], []
     for vid, (name, kw) in enumerate(H1_VARIANTS, start=2):
         m = mjcf.unitree_h1_variant(**kw)
-        js = [j for j in ALL_SPEC_JOINTS if j in m.jnt_names]
-        perm = [int(m.jnt_qposadr[m.jnt_names.index(j)]) for j in js]
-        assert len(perm) == m.nq == m.nv, name
-        up, p = name.upper(), ", ".join(map(str, perm))
-        txt = ("#pragma once\n" + codegen.generate_fk(m, f"om_fk_h1v_{name}") +
-               f"// GENERATED: qpos/qvel address of observation-spec entry k\n"
-               f"__device__ constexpr int OM_H1V_{up}_PERM[{m.nq}] = {{{p}}};\n"
-               f"static const int OM_H1V_{up}_PERM_HOST[{m.nq}] = {{{p}}};\n"
-               f"struct H1V_{name} {{\n"
-               f"  static constexpr int ID = {vid}, NQ = {m.nq}, NBODY = {m.nbody}, NSITE = {m.nsite};\n"
-               f"  static OM_HD int perm(int k) {{ return OM_H1V_{up}_PERM[k]; }}\n"
-               f"  static const int* perm_host() {{ return OM_H1V_{up}_PERM_HOST; }}\n"
-               f"  template <class Sink>\n"
-               f"  static OM_HD void fk(const float (&q)[NQ], const float (&qd)[NQ], Sink& S) {{ om_fk_h1v_{name}(q, qd, S); }}\n"
-               f"}};\n")
-        _write_if_changed(H1V / f"{name}.cuh", txt)
+        _write_if_changed(H1V / f"{name}.cuh", _h1_descriptor(m, name, vid))
         _write_if_changed(H1V / f"tables_{name}.h", "#pragma once\n" + codegen.generate_tables(m, f"om_tab_h1v_{name}"))
         listing.append(f"X({vid}, {name})")
         tables.append(f'#include "tables_{name}.h"\n')
+        if kw.get("hold_weight"):
+            carry_ids.append(vid)
+    carry = mjcf.unitree_h1_variant(hold_weight=True, weight_mass=mjcf.H1_VALID_WEIGHTS[0])
+    body = carry.body_id("weight")
+    _write_if_changed(H1V / f"{H1_CARRY_ENV}.cuh", _h1_descriptor(carry, H1_CARRY_ENV, 0, env_mass_body=body))
     _write_if_changed(H1V / "list.h",
                       "#pragma once\n// GENERATED: (variant id, name) of every UnitreeH1 variant with its own kernels\n"
-                      "#define OM_H1_VARIANTS(X) " + " ".join(listing) + "\n")
+                      "#define OM_H1_VARIANTS(X) " + " ".join(listing) + "\n"
+                      "// the carry variants, whose weight body may take a per-env mass (kernels h1k_carry_env)\n"
+                      "#define OM_H1_IS_CARRY(id) (" + " || ".join(f"(id) == {v}" for v in carry_ids) + ")\n"
+                      f"#define OM_H1_CARRY_WEIGHT_BODY {body}\n")
     _write_if_changed(H1V / "tables.h", "#pragma once\n" + "".join(tables))
 
 
 def compile_units():
-    """(source, extra nvcc flags, object name): every .cu once, and om_traj.cu once more per UnitreeH1 variant."""
+    """(source, extra nvcc flags, object name): every .cu once, and om_traj.cu once more per UnitreeH1 variant (and for
+    the per-env carry kernels)."""
     units = [(src, [], src.stem) for src in sources()]
     units += [(CSRC / "om_traj.cu", [f"-DOM_H1_VARIANT={name}", f'-DOM_H1_VARIANT_HEADER="gen/h1v/{name}.cuh"'],
-               f"om_traj_h1v_{name}") for name, _ in H1_VARIANTS]
+               f"om_traj_h1v_{name}") for name in [n for n, _ in H1_VARIANTS] + [H1_CARRY_ENV]]
     return units
 
 

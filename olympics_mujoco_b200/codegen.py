@@ -238,7 +238,7 @@ def split_parts(model, nparts):
     return parts
 
 
-def generate_fk(model, fn_name, part=None):
+def generate_fk(model, fn_name, part=None, env_mass_body=None):
     """Return CUDA source text of ``template<class Sink> __device__ void <fn_name>(q, qd, S)``.
 
     With ``part=(own_bodies, Exchange)`` the function evaluates only the bodies in ``own_bodies`` and their ancestors,
@@ -246,11 +246,17 @@ def generate_fk(model, fn_name, part=None):
     ``X.com_exchange(sx, sy, sz, 1/M, cx, cy, cz)`` receives this part's sum of m * xipos and returns the normalised total
     (the caller combines the parts -- through shared memory in h1_step_split_kernel).
 
+    With ``env_mass_body=b`` the mass of body ``b`` is a runtime argument, ``<fn_name>(q, qd, S, env_mass)``: its
+    m * xipos term and ``1 / (M0 + env_mass)`` of its tree are emitted instead of folded (M0 = the tree's other bodies).
+    The carried weight of UnitreeH1 is such a body: one function serves every mass.
+
     Sink interface (all indices are literals so unused outputs are dead-code eliminated):
       S.xpos(b,x,y,z)  S.xquat(b,w,x,y,z)  S.site_xpos(s,x,y,z)  S.site_xmat(s,m0..m8)
       S.cvel(b,wx,wy,wz,vx,vy,vz)  S.com(x,y,z)
       S.vel_p(b,wx,wy,wz,vx,vy,vz)   [w; v of the body-fixed point at xpos[rootid]]
     """
+    if env_mass_body is not None and (part is not None or not 0 < env_mass_body < model.nbody):
+        raise ValueError("env_mass_body names one body of a whole-model FK")
     g = Gen()
     nb = model.nbody
     own = set(range(nb)) if part is None else set(part)
@@ -342,7 +348,12 @@ def generate_fk(model, fn_name, part=None):
         # consumer that only needs point velocities (mj_objectVelocity) skip the COM pass entirely
         g.emit(f"S.vel_p({i}, {w_i[0]}, {w_i[1]}, {w_i[2]}, {v_i[0]}, {v_i[1]}, {v_i[2]});")
         m = float(model.body_mass[i])
-        if m > 0:
+        if i == env_mass_body:
+            xi = g.vadd(p, g.qrot(qt, c3(model.body_ipos[i])))
+            acc = com_acc.get(rid, [ZERO, ZERO, ZERO])
+            com_acc[rid] = g.vfma(xi, E(n="env_mass"), acc)
+            com_mass.setdefault(rid, 0.0)
+        elif m > 0:
             xi = g.vadd(p, g.qrot(qt, c3(model.body_ipos[i])))
             acc = com_acc.get(rid, [ZERO, ZERO, ZERO])
             com_acc[rid] = g.vfma(xi, E(m), acc)
@@ -372,8 +383,13 @@ def generate_fk(model, fn_name, part=None):
             g.emit("S.com(com_x, com_y, com_z);")
         dvec[1] = g.vsub(com, P[1])
     else:
+        env_root = None if env_mass_body is None else int(model.body_rootid[env_mass_body])
         for rid, acc in com_acc.items():
-            com = g.vscale(acc, E(1.0 / com_mass[rid]))
+            if rid == env_root:
+                inv = g.tmp(f"1.0f / ({_f(com_mass[rid])} + env_mass)")
+                com = g.vscale(acc, inv)
+            else:
+                com = g.vscale(acc, E(1.0 / com_mass[rid]))
             if rid == 1:
                 g.emit(f"S.com({com[0]}, {com[1]}, {com[2]});")
             dvec[rid] = g.vsub(com, P[rid])
@@ -392,9 +408,12 @@ def generate_fk(model, fn_name, part=None):
             f"(fingerprint {model_fingerprint(model)}) -- do not edit.\n"
             f"// nbody={model.nbody} njnt={model.njnt} nq={model.nq} nv={model.nv} nsite={model.nsite}\n"
             + (f"// part: bodies {sorted(own)}\n" if part is not None else "") +
+            (f"// runtime mass: body {env_mass_body} ({model.body_names[env_mass_body]})\n"
+             if env_mass_body is not None else "") +
             (f"template <class Sink, class Exchange>\n" if part is not None else f"template <class Sink>\n") +
             f"OM_HD void {fn_name}(const float (&q)[{model.nq}], const float (&qd)[{model.nv}], Sink& S"
-            + (", Exchange& X" if part is not None else "") + ") {\n")
+            + (", Exchange& X" if part is not None else "") + (", float env_mass" if env_mass_body is not None else "")
+            + ") {\n")
     return head + body + "\n}\n"
 
 

@@ -104,6 +104,11 @@ struct OmModel {
   int specialised = om::SPEC_NONE;
   int h1_variant = 0;   // UnitreeH1 model with fused playback / live-step kernels: 1 default, 2.. gen/h1v/list.h; else 0
   int device = 0;
+  // om_model_bind_env_body_mass: body env_mass_body's mass is env_mass[env] (device, [env_mass_ld]) in every FK of this
+  // model; env_mass_m0 = the other bodies' mass in its tree.  Null: the tables' mass.
+  const float* env_mass = nullptr;
+  int env_mass_body = -1, env_mass_ld = 0;
+  float env_mass_m0 = 0.f;
 };
 
 #include "om_math.cuh"

@@ -262,6 +262,8 @@ int make_spec(const OmH1Spec* spec, const OmModel* m, H1SpecDev* out) {
   return 0;
 }
 
+static FkEnvMass env_mass_arg(const OmModel* m) { return FkEnvMass{m->env_mass, m->env_mass_body, m->env_mass_m0}; }
+
 }  // namespace om
 
 using namespace om;
@@ -281,8 +283,11 @@ extern "C" int om_fk(const OmModel* m, const float* qpos, const float* qvel, int
     fk_spec_kernel<SPEC_H1, BLOCK><<<grid, BLOCK, 0, st>>>(qpos, qvel, n, ld, o);
   else if (!force_generic && m->specialised == SPEC_A3)
     fk_spec_kernel<SPEC_A3, BLOCK><<<grid, BLOCK, 0, st>>>(qpos, qvel, n, ld, o);
-  else
-    fk_generic_kernel<<<grid, BLOCK, 0, st>>>(m->dev, qpos, qvel, n, ld, o);
+  else if (m->env_mass) {
+    OM_REQUIRE(n <= m->env_mass_ld, "om_fk: %d envs, but the bound body mass holds %d", n, m->env_mass_ld);
+    fk_generic_kernel<true><<<grid, BLOCK, 0, st>>>(m->dev, qpos, qvel, n, ld, o, env_mass_arg(m));
+  } else
+    fk_generic_kernel<false><<<grid, BLOCK, 0, st>>>(m->dev, qpos, qvel, n, ld, o, FkEnvMass{});
   OM_LAUNCHED();
   return 0;
 }
@@ -320,8 +325,12 @@ extern "C" int om_h1_step(const OmModel* m, const OmH1Spec* spec, const float* q
     else h1_step_kernel<BLOCK, false, false, false><<<grid, BLOCK, 0, st>>>(sp, qpos, qvel, prev_x_vel, n, ld, o, obs, reward, absorbing);
     OM_LAUNCHED();
   } else {
-    if (want_fk) {
-      fk_generic_kernel<<<grid, BLOCK, 0, st>>>(m->dev, qpos, qvel, n, ld, o);
+    if (want_fk && m->env_mass) {
+      OM_REQUIRE(n <= m->env_mass_ld, "om_h1_step: %d envs, but the bound body mass holds %d", n, m->env_mass_ld);
+      fk_generic_kernel<true><<<grid, BLOCK, 0, st>>>(m->dev, qpos, qvel, n, ld, o, env_mass_arg(m));
+      OM_LAUNCHED();
+    } else if (want_fk) {
+      fk_generic_kernel<false><<<grid, BLOCK, 0, st>>>(m->dev, qpos, qvel, n, ld, o, FkEnvMass{});
       OM_LAUNCHED();
     }
     h1_obs_kernel<<<grid, BLOCK, 0, st>>>(sp, qpos, qvel, prev_x_vel, n, ld, obs, reward, absorbing);

@@ -12,9 +12,18 @@ struct FkOut {
   float* xpos; float* xquat; float* site_xpos; float* site_xmat; float* cvel; float* com;
 };
 
+// ENV_MASS: body em.body's mass is em.mass[env] (om_model_bind_env_body_mass), its tree's inverse mass 1 / (em.m0 + mass)
+struct FkEnvMass {
+  const float* mass;
+  int body;
+  float m0;
+};
+
+template <bool ENV_MASS>
 __global__ void __launch_bounds__(128) fk_generic_kernel(const ModelTab* __restrict__ gtab,
                                                          const float* __restrict__ qpos,
-                                                         const float* __restrict__ qvel, int n, int ld, FkOut o) {
+                                                         const float* __restrict__ qvel, int n, int ld, FkOut o,
+                                                         FkEnvMass em) {
   __shared__ ModelTab tab;
   {
     const int* src = reinterpret_cast<const int*>(gtab);
@@ -25,6 +34,7 @@ __global__ void __launch_bounds__(128) fk_generic_kernel(const ModelTab* __restr
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= n) return;
   const int nb = tab.nbody;
+  const float env_m = ENV_MASS ? em.mass[env] : 0.f;
 
   float px[MAXB], py[MAXB], pz[MAXB];
   float qw[MAXB], qx[MAXB], qy[MAXB], qz[MAXB];
@@ -105,7 +115,7 @@ __global__ void __launch_bounds__(128) fk_generic_kernel(const ModelTab* __restr
     px[i] = p.x; py[i] = p.y; pz[i] = p.z;
     qw[i] = qt.w; qx[i] = qt.x; qy[i] = qt.y; qz[i] = qt.z;
     wx[i] = w.x; wy[i] = w.y; wz[i] = w.z; vx[i] = v.x; vy[i] = v.y; vz[i] = v.z;
-    const float m = tab.body_mass[i];
+    const float m = (ENV_MASS && i == em.body) ? env_m : tab.body_mass[i];
     V3 xi = p + qrot(qt, V3{tab.body_ipos[3 * i], tab.body_ipos[3 * i + 1], tab.body_ipos[3 * i + 2]});
     cax[rid] = fmaf(xi.x, m, cax[rid]); cay[rid] = fmaf(xi.y, m, cay[rid]); caz[rid] = fmaf(xi.z, m, caz[rid]);
   }
@@ -142,7 +152,7 @@ __global__ void __launch_bounds__(128) fk_generic_kernel(const ModelTab* __restr
   // com - P per tree; a massless tree falls back to its root's position (mj_comPos: xipos)
   for (int i = 1; i < nb; ++i)
     if (tab.body_root[i] == i) {
-      const float im = tab.tree_inv_mass[i];
+      const float im = (ENV_MASS && i == tab.body_root[em.body]) ? 1.f / (em.m0 + env_m) : tab.tree_inv_mass[i];
       if (im > 0.f) { cax[i] = cax[i] * im; cay[i] = cay[i] * im; caz[i] = caz[i] * im; }
       else { cax[i] = px[i]; cay[i] = py[i]; caz[i] = pz[i]; }
       if (i == 1 && o.com) {

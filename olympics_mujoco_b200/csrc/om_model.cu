@@ -160,5 +160,26 @@ extern "C" void om_model_destroy(OmModel* m) {
   delete m;
 }
 
+extern "C" int om_model_bind_env_body_mass(OmModel* m, int body, const float* mass, int ld) {
+  OM_REQUIRE(m && mass, "om_model_bind_env_body_mass: null argument");
+  OM_REQUIRE(OM_H1_IS_CARRY(m->h1_variant),
+             "om_model_bind_env_body_mass: only the UnitreeH1 carry models take a per-env body mass (h1 variant %d)",
+             m->h1_variant);
+  OM_REQUIRE(body == OM_H1_CARRY_WEIGHT_BODY, "om_model_bind_env_body_mass: body %d is not the weight body (%d)", body,
+             OM_H1_CARRY_WEIGHT_BODY);
+  OM_REQUIRE(ld >= 1, "om_model_bind_env_body_mass: ld %d < 1", ld);
+  OM_REQUIRE(!m->env_mass || (m->env_mass == mass && m->env_mass_ld == ld),
+             "om_model_bind_env_body_mass: the model is already bound to another buffer (a binding is for life)");
+  const ModelTab& t = m->host;
+  double m0 = 0.0;
+  for (int i = 1; i < t.nbody; ++i)
+    if (i != body && t.body_root[i] == t.body_root[body]) m0 += t.body_mass[i];
+  m->env_mass = mass;
+  m->env_mass_body = body;
+  m->env_mass_ld = ld;
+  m->env_mass_m0 = (float)m0;
+  return 0;
+}
+
 extern "C" int om_model_is_specialised(const OmModel* m) { return m ? m->specialised : 0; }
 extern "C" int om_model_h1_variant(const OmModel* m) { return m ? m->h1_variant : 0; }

@@ -6,9 +6,12 @@
 //   V::NBODY, V::NSITE
 //   V::perm(k) qpos / qvel address of observation-spec entry k
 //   V::fk(q, qd, sink)  the generated FK of the model
+//   V::ENV_MASS  fk takes one more argument, the env's mass of the carried weight (a carry model bound to a per-env mass
+//                with om_model_bind_env_body_mass: the kernels load it once per thread from PlayArgsEnv / LiveArgs::env_mass)
 // build.py compiles this file once more per variant with -DOM_H1_VARIANT=<name>: such a compilation only instantiates the
 // fused kernels of that variant (H1Kernels h1k_<name>), in parallel with the rest of the build.
 #include <cstdlib>
+#include <type_traits>
 #include <vector>
 
 #include "om_common.cuh"
@@ -112,6 +115,13 @@ struct PlayArgs {
   OmPlayOut o;
   double* obs_moments;   // = o.obs_moments (S1 fused into the playback), or null
 };
+// The playback arguments of a variant whose FK takes the env's weight mass.  A type of its own, so that the kernel parameters
+// of every other variant (and with them their code) stay exactly what they were.
+struct PlayArgsEnv : PlayArgs {
+  const float* env_mass;   // [ld] mass of the carried weight per env
+};
+template <class V>
+using PlayArgsOf = std::conditional_t<V::ENV_MASS, PlayArgsEnv, PlayArgs>;
 
 // observation columns 0-3 (pelvis ty, tilt, list, rotation) are the same root joints in every variant
 OM_HD bool h1_fallen_f(float y, float tilt, float lst, float rot) {
@@ -121,13 +131,27 @@ OM_HD bool h1_fallen_f(float y, float tilt, float lst, float rot) {
          (dr < (-PI / 8)) || (dr > (PI / 8));
 }
 
+// the variant's FK, with the env's body mass when the variant takes one
+template <class V, class Sink>
+OM_HD void v_fk(const float (&q)[V::NQ], const float (&qd)[V::NQ], Sink& S, float mass) {
+  if constexpr (V::ENV_MASS) V::fk(q, qd, S, mass);
+  else V::fk(q, qd, S);
+}
+
+// the env's mass of the carried weight, loaded once per thread (0 and no load for a variant without one)
+template <class V, class A>
+OM_HD float v_env_mass(const A& a, size_t env) {
+  if constexpr (V::ENV_MASS) return a.env_mass[env];
+  else return 0.f;
+}
+
 // One playback step given the sim state; shared by both playback kernels.
 //   qs[NQ] (spec order, double) , dq[NQ] (spec order) -> FK outputs at time slot `slot`
 // STREAM: streaming stores -- the time-parallel kernel (few envs, many steps: +2.5 % there); with 10^6 envs in the
 // one-thread-per-env kernel they measured 1.5 % slower.
 template <class V, bool STREAM>
 OM_HD void play_fk(const double (&qs)[V::NQ], const float (&dq)[V::NQ], const OmPlayOut& o, size_t slot, size_t ld,
-                   size_t env) {
+                   size_t env, float mass) {
   float q[V::NQ], qd[V::NQ];
 #pragma unroll
   for (int k = 0; k < V::NQ; ++k) {
@@ -138,7 +162,7 @@ OM_HD void play_fk(const double (&qs)[V::NQ], const float (&dq)[V::NQ], const Om
                            o.xquat ? o.xquat + slot * (V::NBODY * 4) * ld : nullptr,
                            o.site_xpos ? o.site_xpos + slot * (V::NSITE * 3) * ld : nullptr, nullptr,
                            o.cvel ? o.cvel + slot * (V::NBODY * 6) * ld : nullptr, nullptr, ld, env};
-  V::fk(q, qd, S);
+  v_fk<V>(q, qd, S, mass);
 }
 
 // obs / fallen / reward / integer state of one step from the freshly gathered sample row
@@ -248,7 +272,7 @@ __global__ void __launch_bounds__(256) play_moments_kernel(PlayArgs a, OmPlaySta
 }
 
 template <class V, int BLOCK>
-__global__ void __launch_bounds__(BLOCK) play_h1_seq_kernel(PlayArgs a) {
+__global__ void __launch_bounds__(BLOCK) play_h1_seq_kernel(PlayArgsOf<V> a) {
   constexpr int NQ = V::NQ, K = H1Dims<V>::K, KPAD = H1Dims<V>::KPAD;
   const int env = blockIdx.x * BLOCK + threadIdx.x;
   if (env >= a.n) return;
@@ -264,6 +288,7 @@ __global__ void __launch_bounds__(BLOCK) play_h1_seq_kernel(PlayArgs a) {
     dq[k] = a.s.pending[(NQ + k) * ld + e];
   }
   float pxv = a.s.prev_x_vel[e];
+  const float mass = v_env_mass<V>(a, e);
   float samp[KPAD];
   bool have_samp = false;
   if (a.forced) {
@@ -275,7 +300,7 @@ __global__ void __launch_bounds__(BLOCK) play_h1_seq_kernel(PlayArgs a) {
 #pragma unroll
       for (int k = 0; k < NQ; ++k) cq[k] = fma(a.dt, (double)dq[k], cq[k]);          // :515-519
     }
-    play_fk<V, false>(cq, dq, a.o, (size_t)s, ld, e);                                  // :521-525 / :408-410
+    play_fk<V, false>(cq, dq, a.o, (size_t)s, ld, e, mass);                            // :521-525 / :408-410
     ++st;                                                                            // :532
     const bool wrap = st >= a.t.T;
     if (wrap) {                                                                      // :534-537
@@ -404,7 +429,7 @@ __global__ void __launch_bounds__(256) play_snapshot_kernel(PlayArgs a, OmPlaySt
 // the sequential kernel.  grid = (env tiles, time chunks): 4096 envs x 500 steps become ~300k threads
 // instead of 4096, which is what lets a 4096-env rollout fill the 148 SMs.
 template <class V, int BLOCK>
-__global__ void __launch_bounds__(BLOCK) play_h1_tp_kernel(PlayArgs a, int chunk) {
+__global__ void __launch_bounds__(BLOCK) play_h1_tp_kernel(PlayArgsOf<V> a, int chunk) {
   constexpr int NQ = V::NQ, K = H1Dims<V>::K, KPAD = H1Dims<V>::KPAD;
   pdl_wait();                                    // launched while the snapshot kernel drains
   const int env = blockIdx.x * BLOCK + threadIdx.x;
@@ -414,6 +439,7 @@ __global__ void __launch_bounds__(BLOCK) play_h1_tp_kernel(PlayArgs a, int chunk
   const int T = a.t.T;
   int tr = a.snap.traj_no[e], st = a.snap.step_no[e];
   uint32_t rc = a.snap.reset_count[e];
+  const float mass = v_env_mass<V>(a, e);               // after pdl_wait: the draw of the preceding reset is visible
   // ---- replay the wrap resets that happen before step j0
   int seg_start = 0;
   bool first = true;
@@ -480,7 +506,7 @@ __global__ void __launch_bounds__(BLOCK) play_h1_tp_kernel(PlayArgs a, int chunk
 #pragma unroll
       for (int k = 0; k < NQ; ++k) cq[k] = fma(a.dt, (double)dq[k], cq[k]);
     }
-    play_fk<V, true>(cq, dq, a.o, (size_t)s, ld, e);
+    play_fk<V, true>(cq, dq, a.o, (size_t)s, ld, e, mass);
     ++st;
     const bool wrap = st >= T;
     if (wrap) {
@@ -549,6 +575,7 @@ struct LiveArgs {
   float* qpos; float* qvel;
   float* xpos; float* xquat; float* site_xpos; float* cvel;
   float* obs; float* reward; uint8_t* absorbing; uint8_t* wrapped;
+  const float* env_mass;   // [ld] mass of the carried weight per env (V::ENV_MASS), else unused
 };
 
 // STREAM: streaming stores for the FK outputs (131 072 envs: 34.9 -> 31.8 us = 0.97 of HBM; 1 048 576 envs: 0.261 -> 0.266 ms,
@@ -607,7 +634,7 @@ __global__ void __launch_bounds__(BLOCK) h1_live_step_kernel(LiveArgs a) {
   a.prev_x_vel[e] = samp[NQ];                     // dq_pelvis_tx: emitted row NQ - 2 of UnitreeH1's own spec (checked on the host)
   if (a.xpos || a.xquat || a.site_xpos || a.cvel) {
     SoaSink<false, STREAM> S{a.xpos, a.xquat, a.site_xpos, nullptr, a.cvel, nullptr, ld, e};
-    V::fk(q, qd, S);
+    v_fk<V>(q, qd, S, v_env_mass<V>(a, e));      // after pdl_wait (top of the kernel)
   }
 }
 
@@ -746,6 +773,42 @@ extern "C" int om_traj_next(const OmTraj* t, uint64_t seed, uint32_t env_id0, in
   return 0;
 }
 
+namespace om {
+// The model switch of a MultiMuJoCo reset() (loco_env_base.py:586-599), drawn per env: env i takes model
+// Philox(seed; env_id0 + i, count, STREAM_MODEL_RESET) mod n_models, or (env_id0 + i + count + 1) mod n_models in round
+// robin, and the mass its carried weight has in that model.
+constexpr uint32_t STREAM_MODEL_RESET = 32u;      // utils/philox.py
+constexpr int DRAW_MAX_MODELS = 16;
+struct DrawMasses { float m[DRAW_MAX_MODELS]; };
+
+__global__ void __launch_bounds__(256) h1_draw_models_kernel(uint64_t seed, uint32_t env_id0, uint32_t count, int n_models,
+                                                             int random, DrawMasses masses, int32_t* idx, float* mass, int n) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n) return;
+  const uint32_t env = env_id0 + (uint32_t)e;
+  const int k = random ? to_int(om_draw(seed, env, count, STREAM_MODEL_RESET).x, n_models)
+                       : (int)(((uint64_t)env + count + 1u) % (uint64_t)n_models);
+  idx[e] = k;
+  mass[e] = masses.m[k];
+}
+}  // namespace om
+
+extern "C" int om_h1_draw_models(uint64_t seed, uint32_t env_id0, uint32_t count, int n_models, int random,
+                                 const double* body_mass_host, int32_t* idx, float* mass, int n, void* stream) {
+  OM_REQUIRE(n_models >= 1 && n_models <= DRAW_MAX_MODELS, "om_h1_draw_models: n_models %d outside [1,%d]", n_models,
+             DRAW_MAX_MODELS);
+  OM_REQUIRE(body_mass_host, "om_h1_draw_models: null body_mass_host");
+  OM_REQUIRE(n >= 0, "om_h1_draw_models: n < 0");
+  if (n == 0) return 0;
+  OM_REQUIRE(idx && mass, "om_h1_draw_models: null output");
+  DrawMasses dm = {};
+  for (int k = 0; k < n_models; ++k) dm.m[k] = (float)body_mass_host[k];
+  h1_draw_models_kernel<<<ceil_div(n, 256), 256, 0, (cudaStream_t)stream>>>(seed, env_id0, count, n_models, random ? 1 : 0,
+                                                                            dm, idx, mass, n);
+  OM_LAUNCHED();
+  return 0;
+}
+
 #endif  // !OM_H1_VARIANT
 
 namespace om {
@@ -755,13 +818,16 @@ namespace om {
 struct H1Kernels {
   int nq;                      // observation-spec joints; the trajectory has 2 nq keys
   const int* perm_host;        // [nq] qpos/qvel address of observation-spec entry k
-  int (*play)(const OmTraj* t, PlayArgs& a, bool start_reset, void* stream);
+  int (*play)(const OmTraj* t, const PlayArgs& a, bool start_reset, void* stream, const float* env_mass);
   int (*live)(const LiveArgs& a, void* stream);
 };
 
 template <class V>
-int play_launch(const OmTraj* t, PlayArgs& a, bool start_reset, void* stream) {
+int play_launch(const OmTraj* t, const PlayArgs& args, bool start_reset, void* stream, const float* env_mass) {
   constexpr int BLOCK = PLAY_BLOCK;
+  PlayArgsOf<V> a;
+  static_cast<PlayArgs&>(a) = args;
+  if constexpr (V::ENV_MASS) a.env_mass = env_mass;
   const int n = a.n, n_steps = a.n_steps, ld = a.ld;
   const bool mom = a.obs_moments != nullptr;
   // time-parallel when the env count alone cannot fill the machine (148 SMs x 2048 threads)
@@ -849,6 +915,7 @@ namespace om {
 // other variants are instantiated by the -DOM_H1_VARIANT compilations of this file.
 struct H1Default {
   static constexpr int ID = 1, NQ = 17, NBODY = 21, NSITE = 1;
+  static constexpr bool ENV_MASS = false;
   static OM_HD int perm(int k) { return OM_H1_PERM[k]; }
   template <class Sink>
   static OM_HD void fk(const float (&q)[NQ], const float (&qd)[NQ], Sink& S) { om_fk_unitree_h1(q, qd, S); }
@@ -858,9 +925,12 @@ static const H1Kernels h1k_default = {H1Default::NQ, OM_H1_PERM_HOST, &play_laun
 #define OM_H1_VARIANT_DECL(id, name) extern const H1Kernels h1k_##name;
 OM_H1_VARIANTS(OM_H1_VARIANT_DECL)
 #undef OM_H1_VARIANT_DECL
+extern const H1Kernels h1k_carry_env;    // the carry model with a per-env weight mass (gen/h1v/carry_env.cuh)
 
-// the fused kernels of the model's variant (OmModel::h1_variant), or null
+// the fused kernels of the model's variant (OmModel::h1_variant), or null; a carry model bound to a per-env weight mass
+// launches the carry_env kernels instead
 static const H1Kernels* h1_kernels(const OmModel* m) {
+  if (m->env_mass) return &h1k_carry_env;
   switch (m->h1_variant) {
     case H1Default::ID: return &h1k_default;
 #define OM_H1_VARIANT_CASE(id, name) case id: return &h1k_##name;
@@ -892,8 +962,10 @@ static int play_impl(const OmModel* m, const OmH1Spec* spec, const OmTraj* t, ui
   const bool start_reset = (end_episode_reset & 2) != 0;          // OM_PLAY_START_RESET
   a.n = n; a.ld = ld; a.s = *state; a.snap = *state; a.o = *out; a.forced = forced;
   a.obs_moments = out->obs_moments;
+  OM_REQUIRE(!m->env_mass || n <= m->env_mass_ld, "om_h1_play_from_velocity: %d envs, but the bound body mass holds %d",
+             n, m->env_mass_ld);
   OM_REQUIRE(!a.obs_moments || t->d.psum, "om_h1_play_from_velocity: this trajectory handle has no prefix tables");
-  return hk->play(t, a, start_reset, stream);
+  return hk->play(t, a, start_reset, stream, m->env_mass);
 }
 
 extern "C" int om_h1_play_from_velocity(const OmModel* m, const OmH1Spec* spec, const OmTraj* t, uint64_t seed,
@@ -930,6 +1002,9 @@ extern "C" int om_h1_live_step(const OmModel* m, const OmH1Spec* spec, const OmT
   a.prev_x_vel = state->prev_x_vel;
   a.qpos = out->qpos; a.qvel = out->qvel; a.xpos = out->xpos; a.xquat = out->xquat; a.site_xpos = out->site_xpos;
   a.cvel = out->cvel; a.obs = out->obs; a.reward = out->reward; a.absorbing = out->absorbing; a.wrapped = out->wrapped;
+  a.env_mass = m->env_mass;
+  OM_REQUIRE(!m->env_mass || n <= m->env_mass_ld, "om_h1_live_step: %d envs, but the bound body mass holds %d", n,
+             m->env_mass_ld);
   return hk->live(a, stream);
 }
 #else

@@ -53,7 +53,8 @@ class LocoEnvBase:
     def __init__(self, model, action_spec, observation_spec, collision_groups=None, gamma=0.99, horizon=1000,
                  n_substeps=10, reward_type=None, reward_params=None, traj_params=None, random_start=True,
                  init_step_no=None, timestep=0.001, use_foot_forces=False, use_absorbing_states=True,
-                 n_envs=None, device="cuda", seed=0, env_id0=0, random_env_reset=True, **_ignored_viewer_params):
+                 n_envs=None, device="cuda", seed=0, env_id0=0, random_env_reset=True, per_env_model=False,
+                 **_ignored_viewer_params):
         self._single = n_envs is None
         self.n_envs = 1 if n_envs is None else int(n_envs)
         self._device, self._seed, self._env_id0 = device, int(seed), int(env_id0)
@@ -61,13 +62,22 @@ class LocoEnvBase:
         # xml handle per carried weight -- with one MjData / ObservationHelper each; every reset() switches the env object
         # to the next model, or to a random one.  All n envs of this object share the current model, as the reference's
         # single env does.
+        # per_env_model=True (a subclass's opt-in, e.g. UnitreeH1 per_env_weight): the models differ only in quantities the
+        # kernels read per env at run time, and every reset() draws a model for EACH env (_draw_env_models); one MjData
+        # mirror, device model and observation helper then serve all of them.
         models = list(model) if isinstance(model, (list, tuple)) else [model]
         self._models = models
+        self._per_env_model = bool(per_env_model) and len(models) > 1
         self._timestep, self._n_substeps, self._n_intermediate_steps = timestep, n_substeps, 1
-        self._datas = [BatchedData(m, self.n_envs, device=device) for m in models]
-        self._dms = [Kn.DeviceModel(m) for m in models]
-        self.obs_helpers = [ObservationHelper(observation_spec, m, d, max_joint_velocity=None)
-                            for m, d in zip(models, self._datas)]
+        if self._per_env_model:
+            data = BatchedData(models[0], self.n_envs, device=device)
+            self._datas, self._dms = [data] * len(models), [Kn.DeviceModel(models[0])] * len(models)
+            self.obs_helpers = [ObservationHelper(observation_spec, models[0], data, max_joint_velocity=None)] * len(models)
+        else:
+            self._datas = [BatchedData(m, self.n_envs, device=device) for m in models]
+            self._dms = [Kn.DeviceModel(m) for m in models]
+            self.obs_helpers = [ObservationHelper(observation_spec, m, d, max_joint_velocity=None)
+                                for m, d in zip(models, self._datas)]
         self._current_model_idx, self._random_env_reset, self._model_resets = 0, bool(random_env_reset), 0
         model = models[0]
         self._model, self._data, self._dm, self.obs_helper = model, self._datas[0], self._dms[0], self.obs_helpers[0]
@@ -235,8 +245,11 @@ class LocoEnvBase:
         return self._out(self._modify_observation(self._obs))
 
     def _next_model(self):
-        """The model switch of reset() (MultiMuJoCo :586-599); nothing with a single model.  Decided on the host."""
+        """The model switch of reset() (MultiMuJoCo :586-599); nothing with a single model.  Decided on the host; with
+        per_env_model every env also draws its own model on the device (the host's pick is env 0's)."""
         if len(self._models) > 1:
+            if self._per_env_model:
+                self._draw_env_models(self._model_resets)
             if self._random_env_reset:
                 # np.random.randint in the reference; here the Philox contract (stream 32, counter = number of resets)
                 from ..utils.philox import STREAM_MODEL_RESET, philox_randint
@@ -247,7 +260,13 @@ class LocoEnvBase:
             self._model_resets += 1
             self._select_model(self._current_model_idx)
 
+    def _draw_env_models(self, count):
+        raise NotImplementedError
+
     def _select_model(self, idx):
+        if self._per_env_model:               # the one data / device model / helper serve every env's model
+            self._model = self._models[idx]
+            return
         prev = self._data
         self._model, self._data = self._models[idx], self._datas[idx]
         self._dm, self.obs_helper = self._dms[idx], self.obs_helpers[idx]

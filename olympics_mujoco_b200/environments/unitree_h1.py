@@ -69,10 +69,20 @@ class UnitreeH1(BaseHumanoidRobot):
                                      non_combinable=[("carry", None, "perfect")])
 
     def __init__(self, disable_arms=True, disable_back_joint=False, hold_weight=False, weight_mass=None, xml_path=None,
-                 **kwargs):
+                 per_env_weight=False, **kwargs):
         """UnitreeH1.py:38-111.  ``hold_weight``: a jointless "weight" body under torso_link (arms fixed in their MJCF
         orientation); ``weight_mass=None`` builds one model per valid weight (0.1, 1, 5, 10 kg) and every reset() switches
-        the env object to one of them (MultiMuJoCo)."""
+        the env object to one of them (MultiMuJoCo).
+
+        ``per_env_weight=True`` (extension; needs ``hold_weight`` and no fixed ``weight_mass``): every reset() draws a
+        weight for EACH env, as n reference env objects would -- env ``env_id0 + e`` after the object's reset number k
+        holds model ``philox_randint(seed, env_id0 + e, k, 32, 4)`` (``random_env_reset``) or ``(env_id0 + e + k + 1) mod
+        4`` (round robin); env 0 of the first shard follows the shared pick.  ``model_index`` (int32 [n], into
+        ``mjcf.H1_VALID_WEIGHTS``) and ``weight_body_mass`` (float32 [n], 2 x the weight in kg) hold the draw on the device
+        and every kernel of the env reads the mass per env.  Trajectory wrap resets inside an episode keep the weight."""
+        if per_env_weight and (not hold_weight or weight_mass is not None):
+            raise ValueError("per_env_weight draws one of the valid weights per env: it needs hold_weight=True and "
+                             "weight_mass=None")
         if hold_weight:
             assert disable_arms is True, ("If you want Unitree H1 to carry a weight, please disable the arms. "
                                           "They will be kept fixed.")
@@ -89,8 +99,11 @@ class UnitreeH1(BaseHumanoidRobot):
         base = mjcf.compile_mjcf(xml_path, name="UnitreeH1") if xml_path is not None else None   # the user's h1.xml
         weights = [None] if not hold_weight else ([weight_mass] if weight_mass is not None else self._valid_weights)
         models = [mjcf.unitree_h1_variant(disable_arms, disable_back_joint, hold_weight, w, base=base) for w in weights]
-        super().__init__(models if len(models) > 1 else models[0], action_spec, observation_spec, **kwargs)
+        super().__init__(models if len(models) > 1 else models[0], action_spec, observation_spec,
+                         per_env_model=per_env_weight, **kwargs)
         model = self._model
+        if per_env_weight:
+            self._bind_env_weights()
         js = [e[1] for e in observation_spec if e[2] == ObservationType.JOINT_POS]
         perm = [int(model.jnt_qposadr[model.jnt_names.index(j)]) for j in js]
         rf = self._reward_function
@@ -99,6 +112,22 @@ class UnitreeH1(BaseHumanoidRobot):
                                      use_absorbing_states=kwargs.get("use_absorbing_states", True))
         self._fused_reward = hasattr(rf, "_target_vel")
         self._prev_x_vel = torch.zeros(self.n_envs, device=self._device)
+
+    # ------------------------------------------------------------------ per-env carried weight
+    def _bind_env_weights(self):
+        """One device model for the four carry models, its weight body's mass read per env from ``weight_body_mass``.
+        Before the first reset every env holds model 0, as the shared env object does."""
+        if not self._dm.h1_variant:
+            raise NotImplementedError("per_env_weight needs the carry models of the shipped tables (no xml_path)")
+        self._weight_body = self._models[0].body_id("weight")
+        self._weight_masses = [float(m.body_mass[self._weight_body]) for m in self._models]
+        self.model_index = torch.zeros(self.n_envs, dtype=torch.int32, device=self._device)
+        self.weight_body_mass = torch.full((self.n_envs,), self._weight_masses[0], dtype=torch.float32, device=self._device)
+        Kn.bind_env_body_mass(self._dm, self._weight_body, self.weight_body_mass)
+
+    def _draw_env_models(self, count):
+        Kn.h1_draw_models(self._seed, self._env_id0, count, self._weight_masses, self.model_index, self.weight_body_mass,
+                          random=self._random_env_reset)
 
     # ------------------------------------------------------------------ specs (UnitreeH1.py:134-160, 293-376)
     def _get_xml_modifications(self):

@@ -90,6 +90,24 @@ class DeviceModel:
             pass
 
 
+def bind_env_body_mass(dm: DeviceModel, body, mass):
+    """``om_model_bind_env_body_mass``: from now on every FK of ``dm`` (a UnitreeH1 carry model) reads body ``body``'s mass
+    of env i from ``mass[i]`` (float32 [n] CUDA tensor, updated in place by its owner).  For the model's life: the tensor
+    is kept alive by ``dm``."""
+    check(_lib.load().om_model_bind_env_body_mass(dm.handle, int(body), _p(mass, torch.float32), max(mass.numel(), 1)))
+    dm.env_mass = mass
+
+
+def h1_draw_models(seed, env_id0, count, body_masses, idx, mass, random=True):
+    """``om_h1_draw_models``: the per-env model switch of one MultiMuJoCo reset (counter ``count``) into ``idx`` (int32
+    [n]) and ``mass`` (float32 [n], ``body_masses[idx]``), on the device, in place."""
+    bm = np.ascontiguousarray(body_masses, dtype=np.float64)
+    n = idx.numel()
+    assert mass.numel() == n
+    check(_lib.load().om_h1_draw_models(int(seed), int(env_id0), int(count), len(bm), int(bool(random)), bm.ctypes.data,
+                                        _p(idx, torch.int32), _p(mass, torch.float32), n, _stream()))
+
+
 def fk(dm: DeviceModel, qpos, qvel=None, want=("xpos", "xquat", "site_xpos", "site_xmat", "cvel", "subtree_com"),
        force_generic=False, out=None):
     """K1.  qpos [nq,n], qvel [nv,n] -> dict of SoA tensors."""

@@ -22,3 +22,13 @@ def philox_randint(seed, env_id, count, stream, n):
     seed = int(seed)
     w = philox4x32_10((env_id, count, stream, 0), (seed & _MASK, (seed >> 32) & _MASK))
     return (w[0] * int(n)) >> 32
+
+
+def env_model_draw(seed, env_id, count, n_models, random=True):
+    """The model that env ``env_id`` (global id) holds after its env object's reset number ``count`` (0-based) when every
+    env draws its own (``per_env_weight``; ``om_h1_draw_models`` on the device): random -- the shared draw keyed on the env
+    instead of the object; round robin -- model ``(env_id + count + 1) mod n_models``.  Env id 0 follows the sequence a
+    shared MultiMuJoCo env object picks."""
+    if random:
+        return philox_randint(seed, env_id, count, STREAM_MODEL_RESET, n_models)
+    return (int(env_id) + int(count) + 1) % int(n_models)

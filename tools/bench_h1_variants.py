@@ -3,6 +3,10 @@ process, alternating: fused play_trajectory_from_velocity at 4096 envs x 500 ste
 reward, fallen, trajectory state), one call of the base class's per-step path at the same size, and step_graph replay time
 per step at 131 072 envs.  One JSON line (measurement aid).
 
+``carry_per_env`` is the carry task with a weight drawn per env (``per_env_weight=True``: every env of the batch carries its
+own of the four weights, the kernels read its mass at run time); it alternates with the fixed 1 kg carry kernels
+(``carry_1``) like every other row.  Its call time includes the two model draws of the call (start and end reset).
+
 Algorithmic bytes per env-step, from shapes: 2 NQ * 4 sample in + nbody * 13 * 4 FK out (xpos, xquat, cvel) + nsite * 12
 + (2 NQ - 2) * 4 obs + 13 (reward, fallen, traj_no, step_no) + 2 NQ * 4 (the carried / reset sample)."""
 import argparse
@@ -20,7 +24,8 @@ WANT = ("xpos", "xquat", "site_xpos", "cvel", "obs", "reward", "fallen", "traj_n
 VARIANTS = dict(default={}, noback=dict(disable_back_joint=True), arms=dict(disable_arms=False),
                 arms_noback=dict(disable_arms=False, disable_back_joint=True),
                 carry_0p1=dict(hold_weight=True, weight_mass=0.1), carry_1=dict(hold_weight=True, weight_mass=1.0),
-                carry_5=dict(hold_weight=True, weight_mass=5.0), carry_10=dict(hold_weight=True, weight_mass=10.0))
+                carry_5=dict(hold_weight=True, weight_mass=5.0), carry_10=dict(hold_weight=True, weight_mass=10.0),
+                carry_per_env=dict(hold_weight=True, per_env_weight=True))
 
 
 def bytes_per_env_step(m):
@@ -31,7 +36,8 @@ def bytes_per_env_step(m):
 def make_env(kw, n):
     import olympics_mujoco_b200 as om
     from olympics_mujoco_b200 import mjcf, synthetic
-    model = mjcf.unitree_h1_variant(**kw)
+    model = mjcf.unitree_h1_variant(**{k: v for k, v in kw.items() if k != "per_env_weight"},
+                                    **({"weight_mass": 1.0} if kw.get("per_env_weight") else {}))
     data = synthetic.h1_walk_dataset(n_traj=4, t_raw=2500, seed=1, model=model)
     return om.LocoEnvBase.make("UnitreeH1.walk.real", n_envs=n, seed=3, **kw,
                                traj_params=dict(traj_files=data, traj_dt=1 / 500, control_dt=0.01))
