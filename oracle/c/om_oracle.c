@@ -220,69 +220,114 @@ static int h1_has_fallen(const double* obs) {
          (obs[2] < -PI / 12) || (obs[2] > PI / 8) || (obs[3] < (-PI / 8)) || (obs[3] > (PI / 8));
 }
 
-/* play_trajectory_from_velocity for n_env envs, one episode of n_steps (loco_env_base.py:444-560), the
- * initial reset included.  table [K][n_traj][T] float64.  Outputs (any may be NULL) are env-major
- * [n_env][n_steps][...]; `checksum` [n_env] always receives a sum over everything computed, so that a
- * timing run without outputs cannot be optimised away. */
-void or_h1_play(const OrModel* m, const int* perm, const double* table, int K, int n_traj, int T, uint64_t seed,
-                uint32_t env_id0, int n_env, int n_steps, double dt, double target, double* xpos, double* xquat,
-                double* site_xpos, double* cvel, double* obs, double* reward, uint8_t* fallen, int32_t* traj_no_t,
-                int32_t* step_no_t, double* checksum) {
+/* What one env carries from one playback call to the next (the device's OmPlayState), env-major: traj_no, step_no,
+ * reset_count [n_env]; xy_off [n_env][2]; curr_qpos [n_env][K/2]; pending [n_env][K], the loop's `sample` variable
+ * (x, y re-centred), which stays the stale one across the end-of-episode reset; prev_x_vel [n_env], dq_pelvis_tx of
+ * the previous observation. */
+typedef struct {
+  int32_t *traj_no, *step_no;
+  uint32_t* reset_count;
+  double *xy_off, *curr_qpos, *pending, *prev_x_vel;
+} OrPlayState;
+
+/* play_trajectory_from_velocity for the envs env_id0 .. env_id0 + n_env - 1: n_episodes episodes of n_steps
+ * (loco_env_base.py:444-560), each ending with reset() (:555-557).  start_reset: the call begins with reset()
+ * (:481-508); 0 carries the state of the previous call on (the device's continue_episode).  `ps` is read at the start
+ * and written at the end; NULL = a fresh env (reset_count 0, start_reset required) whose final state is dropped.
+ * table [K][n_traj][T] float64.  Outputs (any may be NULL) are env-major [n_env][n_episodes * n_steps][...];
+ * `checksum` [n_env] always receives a sum over everything computed, so that a timing run without outputs cannot be
+ * optimised away. */
+void or_h1_play_chain(const OrModel* m, const int* perm, const double* table, int K, int n_traj, int T, uint64_t seed,
+                      uint32_t env_id0, int n_env, int n_episodes, int n_steps, int start_reset, double dt, double target,
+                      const OrPlayState* ps, double* xpos, double* xquat, double* site_xpos, double* cvel, double* obs,
+                      double* reward, uint8_t* fallen, int32_t* traj_no_t, int32_t* step_no_t, double* checksum) {
   const int nj = K / 2, nb = m->nbody;
+  const size_t n_slots = (size_t)n_episodes * n_steps;
 #pragma omp parallel for schedule(static)
   for (int e = 0; e < n_env; ++e) {
     double sample[64], curr[32], qpos[MAXV], qvel[MAXV], bx[MAXB * 3], bq[MAXB * 4], bs[24], bc[MAXB * 6], ob[64];
-    int tr, st;
-    uint32_t rc = 0;
-    double ox, oy, acc = 0.0, prev_xv;
+    int tr = 0, st = 0;
+    uint32_t rc = ps ? ps->reset_count[e] : 0;
+    double ox = 0.0, oy = 0.0, acc = 0.0, prev_xv = 0.0;
 #define TAB(k, tr_, s_) table[((size_t)(k) * n_traj + (tr_)) * T + (s_)]
 #define LOAD_SAMPLE()                                                          \
   do {                                                                         \
     for (int k = 0; k < K; ++k) sample[k] = TAB(k, tr, st);                    \
     sample[0] -= ox; sample[1] -= oy;                                          \
   } while (0)
-    traj_draw(seed, env_id0 + e, rc++, n_traj, T, &tr, &st);                    /* :481 reset() */
-    ox = TAB(0, tr, st); oy = TAB(1, tr, st);
-    LOAD_SAMPLE();                                                              /* :483 */
-    prev_xv = sample[nj];                                                       /* obs[15] of reset() */
-    for (int k = 0; k < nj; ++k) curr[k] = sample[k];                           /* :508 */
-    for (int s = 0; s < n_steps; ++s) {
-      for (int k = 0; k < nj; ++k) {                                            /* :515-521 */
-        const double qs = curr[k] + dt * sample[nj + k];
-        qpos[perm[k]] = qs; qvel[perm[k]] = sample[nj + k];
-        curr[k] = qs;                                                           /* :529 */
+    if (start_reset || !ps) {
+      traj_draw(seed, env_id0 + e, rc++, n_traj, T, &tr, &st);                  /* :481 reset() */
+      ox = TAB(0, tr, st); oy = TAB(1, tr, st);
+      LOAD_SAMPLE();                                                            /* :483 */
+      prev_xv = sample[nj];                                                     /* obs[15] of reset() */
+      for (int k = 0; k < nj; ++k) curr[k] = sample[k];                         /* :508 */
+    } else {
+      tr = ps->traj_no[e]; st = ps->step_no[e];
+      ox = ps->xy_off[2 * e]; oy = ps->xy_off[2 * e + 1];
+      memcpy(sample, ps->pending + (size_t)e * K, sizeof(double) * K);
+      memcpy(curr, ps->curr_qpos + (size_t)e * nj, sizeof(double) * nj);
+      prev_xv = ps->prev_x_vel[e];
+    }
+    for (int ep = 0; ep < n_episodes; ++ep) {
+      for (int s = 0; s < n_steps; ++s) {
+        for (int k = 0; k < nj; ++k) {                                          /* :515-521 */
+          const double qs = curr[k] + dt * sample[nj + k];
+          qpos[perm[k]] = qs; qvel[perm[k]] = sample[nj + k];
+          curr[k] = qs;                                                         /* :529 */
+        }
+        or_forward(m, qpos, qvel, bx, bq, bs, 0, bc, 0);                        /* :525 mj_forward subset */
+        const size_t slot = (size_t)e * n_slots + (size_t)ep * n_steps + s;
+        if (xpos) memcpy(xpos + slot * nb * 3, bx, sizeof(double) * nb * 3);
+        if (xquat) memcpy(xquat + slot * nb * 4, bq, sizeof(double) * nb * 4);
+        if (site_xpos) memcpy(site_xpos + slot * m->nsite * 3, bs, sizeof(double) * m->nsite * 3);
+        if (cvel) memcpy(cvel + slot * nb * 6, bc, sizeof(double) * nb * 6);
+        acc += bx[3 * (nb - 1)] + bq[4 * (nb - 1)] + bc[6 * (nb - 1) + 3];
+        ++st;                                                                   /* :532 */
+        if (st == T) {                                                          /* :534-537 */
+          traj_draw(seed, env_id0 + e, rc++, n_traj, T, &tr, &st);
+          ox = TAB(0, tr, st); oy = TAB(1, tr, st);
+          LOAD_SAMPLE();
+          for (int k = 0; k < nj; ++k) curr[k] = sample[k];
+        } else {
+          LOAD_SAMPLE();
+        }
+        for (int k = 0; k < K - 2; ++k) ob[k] = sample[k + 2];                  /* :539 */
+        const int f = h1_has_fallen(ob);                                        /* :541 */
+        const double r = exp(-(prev_xv - target) * (prev_xv - target));         /* reward.py:72-74 on the previous obs */
+        prev_xv = ob[nj - 2];
+        if (obs) memcpy(obs + slot * (K - 2), ob, sizeof(double) * (K - 2));
+        if (reward) reward[slot] = r;
+        if (fallen) fallen[slot] = (uint8_t)f;
+        if (traj_no_t) traj_no_t[slot] = tr;
+        if (step_no_t) step_no_t[slot] = st;
+        acc += r + f + ob[0];
       }
-      or_forward(m, qpos, qvel, bx, bq, bs, 0, bc, 0);                          /* :525 mj_forward subset */
-      const size_t slot = (size_t)e * n_steps + s;
-      if (xpos) memcpy(xpos + slot * nb * 3, bx, sizeof(double) * nb * 3);
-      if (xquat) memcpy(xquat + slot * nb * 4, bq, sizeof(double) * nb * 4);
-      if (site_xpos) memcpy(site_xpos + slot * m->nsite * 3, bs, sizeof(double) * m->nsite * 3);
-      if (cvel) memcpy(cvel + slot * nb * 6, bc, sizeof(double) * nb * 6);
-      acc += bx[3 * (nb - 1)] + bq[4 * (nb - 1)] + bc[6 * (nb - 1) + 3];
-      ++st;                                                                     /* :532 */
-      if (st == T) {                                                            /* :534-537 */
-        traj_draw(seed, env_id0 + e, rc++, n_traj, T, &tr, &st);
-        ox = TAB(0, tr, st); oy = TAB(1, tr, st);
-        LOAD_SAMPLE();
-        for (int k = 0; k < nj; ++k) curr[k] = sample[k];
-      } else {
-        LOAD_SAMPLE();
-      }
-      for (int k = 0; k < K - 2; ++k) ob[k] = sample[k + 2];                    /* :539 */
-      const int f = h1_has_fallen(ob);                                          /* :541 */
-      const double r = exp(-(prev_xv - target) * (prev_xv - target));           /* reward.py:72-74 on the previous obs */
-      prev_xv = ob[nj - 2];
-      if (obs) memcpy(obs + slot * (K - 2), ob, sizeof(double) * (K - 2));
-      if (reward) reward[slot] = r;
-      if (fallen) fallen[slot] = (uint8_t)f;
-      if (traj_no_t) traj_no_t[slot] = tr;
-      if (step_no_t) step_no_t[slot] = st;
-      acc += r + f + ob[0];
+      traj_draw(seed, env_id0 + e, rc++, n_traj, T, &tr, &st);                  /* :555 reset(); `sample` stays stale */
+      ox = TAB(0, tr, st); oy = TAB(1, tr, st);
+      curr[0] = 0.0; curr[1] = 0.0;                                             /* :557, x and y re-centred: exactly 0 */
+      for (int k = 2; k < nj; ++k) curr[k] = TAB(k, tr, st);
+      prev_xv = TAB(nj, tr, st);
     }
     checksum[e] = acc;
+    if (ps) {
+      ps->traj_no[e] = tr; ps->step_no[e] = st; ps->reset_count[e] = rc;
+      ps->xy_off[2 * e] = ox; ps->xy_off[2 * e + 1] = oy;
+      memcpy(ps->pending + (size_t)e * K, sample, sizeof(double) * K);
+      memcpy(ps->curr_qpos + (size_t)e * nj, curr, sizeof(double) * nj);
+      ps->prev_x_vel[e] = prev_xv;
+    }
 #undef TAB
 #undef LOAD_SAMPLE
   }
+}
+
+/* One episode of n_steps from a fresh reset for each env (outputs [n_env][n_steps][...]): the CPU baseline's call. */
+void or_h1_play(const OrModel* m, const int* perm, const double* table, int K, int n_traj, int T, uint64_t seed,
+                uint32_t env_id0, int n_env, int n_steps, double dt, double target, double* xpos, double* xquat,
+                double* site_xpos, double* cvel, double* obs, double* reward, uint8_t* fallen, int32_t* traj_no_t,
+                int32_t* step_no_t, double* checksum) {
+  or_h1_play_chain(m, perm, table, K, n_traj, T, seed, env_id0, n_env, 1, n_steps, 1, dt, target, 0, xpos, xquat,
+                   site_xpos, cvel, obs, reward, fallen, traj_no_t, step_no_t, checksum);
 }
 
 /* ---------------------------------------------------------------- compute_gae per env over [n_env][T] (env-major) */

@@ -22,8 +22,9 @@ class OrModel(C.Structure):
 def lib():
     global _lib
     if _lib is None:
-        if not LIB.exists():
-            subprocess.check_call(["make", "-s", "-C", str(DIR)])
+        # every time, not only when the .so is missing: a no-op when it is up to date, and a stale library would
+        # otherwise test the old C code
+        subprocess.check_call(["make", "-s", "-C", str(DIR)])
         _lib = C.CDLL(str(LIB))
         _lib.or_num_threads.restype = C.c_int
     return _lib
@@ -60,8 +61,8 @@ def forward(cm, qpos, qvel):
 
 
 def h1_play_buffers(km, K, n_env, n_steps):
-    """Output arrays of ``h1_play(record=True)``; allocate once and pass as ``out=`` to keep page faults and zero
-    fills out of a timed region."""
+    """Output arrays of ``h1_play(record=True)`` (``n_steps``: all episodes' steps); allocate once and pass as ``out=`` to
+    keep page faults and zero fills out of a timed region."""
     return dict(xpos=np.zeros((n_env, n_steps, km.nbody * 3)), xquat=np.zeros((n_env, n_steps, km.nbody * 4)),
                 site_xpos=np.zeros((n_env, n_steps, km.nsite * 3)), cvel=np.zeros((n_env, n_steps, km.nbody * 6)),
                 obs=np.zeros((n_env, n_steps, K - 2)), reward=np.zeros((n_env, n_steps)),
@@ -69,19 +70,49 @@ def h1_play_buffers(km, K, n_env, n_steps):
                 step_no=np.zeros((n_env, n_steps), np.int32), checksum=np.zeros(n_env))
 
 
-def h1_play(cm, perm, table, seed, env_id0, n_env, n_steps, dt=0.01, target=1.25, record=True, out=None):
+class OrPlayState(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("traj_no", "step_no", "reset_count", "xy_off", "curr_qpos", "pending",
+                                          "prev_x_vel")]
+
+
+def play_state(K, n_env):
+    """The per-env state one playback call hands the next (the device's OmPlayState), env-major, float64 where the
+    device keeps float32: traj_no, step_no, reset_count [n_env], xy_off [n_env, 2], curr_qpos [n_env, K/2], pending
+    [n_env, K] (the loop's stale ``sample``), prev_x_vel [n_env].  All zero = a fresh env; its first call must reset."""
+    return dict(traj_no=np.zeros(n_env, np.int32), step_no=np.zeros(n_env, np.int32),
+                reset_count=np.zeros(n_env, np.uint32), xy_off=np.zeros((n_env, 2)), curr_qpos=np.zeros((n_env, K // 2)),
+                pending=np.zeros((n_env, K)), prev_x_vel=np.zeros(n_env))
+
+
+def h1_play(cm, perm, table, seed, env_id0, n_env, n_steps, dt=0.01, target=1.25, record=True, out=None, n_episodes=1,
+            state=None, start_reset=True):
+    """``play_trajectory_from_velocity`` for envs ``env_id0 ..`` ``env_id0 + n_env - 1``: ``n_episodes`` episodes of
+    ``n_steps``, each ending with reset() (outputs [n_env, n_episodes * n_steps, ...]).  ``state`` (``play_state``) is
+    read at the start and updated in place; ``None`` = fresh envs, final state dropped.  ``start_reset=False`` continues
+    the state's episode instead of beginning with reset()."""
     km = cm.km
     table = np.ascontiguousarray(table, np.float64)
     K, n_traj, T = table.shape
     perm = np.ascontiguousarray(perm, np.int32)
+    n_slots = n_episodes * n_steps
     if out is None:
-        out = h1_play_buffers(km, K, n_env, n_steps) if record else dict(checksum=np.zeros(n_env))
+        out = h1_play_buffers(km, K, n_env, n_slots) if record else dict(checksum=np.zeros(n_env))
     else:
-        assert out["reward"].shape == (n_env, n_steps)
+        assert out["checksum"].shape == (n_env,) and ("reward" not in out or out["reward"].shape == (n_env, n_slots))
+    if state is None:
+        assert start_reset, "a fresh env begins with reset()"
+        ps = None
+    else:
+        want = play_state(K, n_env)
+        for k, v in want.items():
+            a = state[k]
+            assert isinstance(a, np.ndarray) and a.shape == v.shape and a.dtype == v.dtype and a.flags.c_contiguous, k
+        ps = C.byref(OrPlayState(**{k: state[k].ctypes.data for k in want}))
     g = lambda k: _p(out.get(k))
-    lib().or_h1_play(C.byref(cm.c), _p(perm), _p(table), K, n_traj, T, C.c_uint64(seed), C.c_uint32(env_id0), n_env, n_steps,
-                     C.c_double(dt), C.c_double(target), g("xpos"), g("xquat"), g("site_xpos"), g("cvel"), g("obs"),
-                     g("reward"), g("fallen"), g("traj_no"), g("step_no"), _p(out["checksum"]))
+    lib().or_h1_play_chain(C.byref(cm.c), _p(perm), _p(table), K, n_traj, T, C.c_uint64(seed), C.c_uint32(env_id0), n_env,
+                           n_episodes, n_steps, int(bool(start_reset)), C.c_double(dt), C.c_double(target), ps, g("xpos"),
+                           g("xquat"), g("site_xpos"), g("cvel"), g("obs"), g("reward"), g("fallen"), g("traj_no"),
+                           g("step_no"), _p(out["checksum"]))
     return out
 
 

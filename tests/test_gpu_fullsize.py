@@ -1,6 +1,9 @@
-"""GPU tests at BASELINE.json's FULL sizes, through size-independent properties (the oracle is far too slow there):
+"""GPU tests at BASELINE.json's FULL sizes through size-independent properties and kernel-against-kernel agreement:
 configs[1] 4096 envs x 500 steps H1 playback, configs[2] 16384 envs x 64 steps A3 rollout, configs[4] 1 M sharded envs.
-(configs[3], the 65536-env discriminator, is covered against the oracle in test_gpu_disc.py.)"""
+The time-parallel and sequential playback kernels compared here share their loop body, so a defect common to both
+passes; test_gpu_fullsize_oracle.py compares the benchmarked configs[1] step and a configs[4] shard with the float64 C
+oracle on every env and step.  (configs[3], the 65536-env discriminator, is covered against the oracle in
+test_gpu_disc.py.)"""
 import numpy as np
 import pytest
 
