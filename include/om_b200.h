@@ -298,9 +298,13 @@ int om_a3_reset(const OmModel* m, const OmA3Task* task, uint64_t seed, uint32_t 
  * K4: discriminator reward  r = -log(1 - sigmoid(D(s)) + 1e-8)  (GAIL.make_discrim_reward,
  * imitation_lib/imitation/gail_TRPO.py:320-327; VAIL discrim_output vail_TRPO.py:18-21) for the two networks
  * the reference configures for UnitreeH1 (examples/imitation_learning/utils.py:151-179, confs.yaml:113-130):
- *   kind 0 VAIL  VariationalNet (networks.py:258-284): 32 -relu-> 256 -relu-> 128 -> mu[128], logvar[128],
+ *   kind 0 VAIL  VariationalNet (networks.py:258-284): n_in -relu-> 256 -relu-> 128 -> mu[128], logvar[128],
  *                z = mu + exp(logvar/2) * eps (:21-24), d = wd . z + bd
- *   kind 1 GAIL  DiscriminatorNetwork (:208-234): 32 -tanh-> 512 -tanh-> 256 -> 1
+ *   kind 1 GAIL  DiscriminatorNetwork (:208-234): n_in -tanh-> 512 -tanh-> 256 -> 1
+ * n_in = 1..64: the kinematic observation of the env's UnitreeH1 variant (env.get_kinematic_obs_mask(): 32 for the
+ * default model and the carry task, 30 without the back joint, 48 with arms, 46 with arms and without the back joint);
+ * other values are refused.  The kernel variants forced through the "disc_vail2" / "disc_pg2" knobs (om_debug_set)
+ * take n_in = 32 only: with another width om_disc_reward / om_disc_forward fail (om_last_error) and launch nothing.
  * Weights are HOST pointers, row-major [out][in] float32 (torch.nn.Linear.weight), copied at create time.
  * The contraction runs on tcgen05 tensor cores as 3xTF32 with fp32 accumulation (fp32-level results). */
 typedef struct OmDiscDesc {

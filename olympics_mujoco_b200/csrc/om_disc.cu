@@ -150,6 +150,24 @@ struct DiscArgs {
   int n, ld;
 };
 
+// Input width of the default kernels (disc_vail4_kernel, disc_reward_pg2_kernel).  IN = 0 is the build for the default
+// H1 observation: 32 inputs, one 32-column input chunk, DiscArgs.  IN = 1 / 2 serve any other width n_in <= 32 IN: one /
+// two input chunks, n_in given at run time in a derived argument type (so that the 32-input kernels keep their
+// parameters), input rows at or beyond n_in never read and their standardised value 0 (the host image gives the padding
+// columns of W1 zero weights).
+constexpr int DISC_MAX_IN = 64;
+struct DiscArgsIn : DiscArgs { int n_in; };
+template <int IN> struct DiscInput {
+  using Args = DiscArgsIn;
+  static constexpr int NCH = IN;                // 32-column input chunks
+  __device__ static int n_in(const Args& a) { return a.n_in; }
+};
+template <> struct DiscInput<0> {
+  using Args = DiscArgs;
+  static constexpr int NCH = 1;
+  __device__ static int n_in(const Args&) { return DISC_IN; }
+};
+
 enum { ACT_RELU = 0, ACT_TANH = 1 };
 template <int ACT> __device__ __forceinline__ float act(float x) { return ACT == ACT_RELU ? fmaxf(x, 0.f) : tanhf(x); }
 
@@ -419,8 +437,8 @@ __device__ __forceinline__ void store_a_half(uint8_t* stage, int row, int half, 
   }
 }
 
-template <int N1, int N2, bool VAIL, bool KL>
-__global__ void __launch_bounds__(320, 1) disc_reward_pg2_kernel(DiscArgs a) {
+template <int N1, int N2, bool VAIL, bool KL, int IN = 0>
+__global__ void __launch_bounds__(320, 1) disc_reward_pg2_kernel(typename DiscInput<IN>::Args a) {
   constexpr int ACT = VAIL ? ACT_RELU : ACT_TANH;
   constexpr int NB1 = N1 / 256;
   constexpr int Z = 128;
@@ -428,7 +446,10 @@ __global__ void __launch_bounds__(320, 1) disc_reward_pg2_kernel(DiscArgs a) {
   constexpr int D1_COL = 0, D2_COL = 256, D3_COL = 0;
   constexpr int HEAD_K = VAIL ? Z : N2;
   constexpr int NPROD = 256;
+  constexpr int NCH = DiscInput<IN>::NCH, KIN = KC * NCH;            // input chunks, padded input width
   static_assert(N1 % 256 == 0 && N2 % 32 == 0 && N2 <= 256, "unsupported discriminator shape");
+  static_assert(DISC_MAX_PAR - 2 * KIN >= N1 + N2 + (VAIL ? N3 : 0) + HEAD_K + 1, "standardiser slots overlap the parameters");
+  const int nin = DiscInput<IN>::n_in(a);
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* stA = smem;
   uint8_t* stB = smem + 2 * STAGE_A_BYTES;
@@ -449,9 +470,13 @@ __global__ void __launch_bounds__(320, 1) disc_reward_pg2_kernel(DiscArgs a) {
 
   constexpr int NPAR = N1 + N2 + (VAIL ? N3 : 0) + HEAD_K + 1;
   for (int i = tid; i < NPAR; i += 320) par[i] = a.params[i];
-  float* s_mean = par + DISC_MAX_PAR - 2 * DISC_IN;
-  float* s_inv = s_mean + DISC_IN;
-  if (tid < DISC_IN) { s_mean[tid] = a.mean[tid]; s_inv[tid] = 1.0f / a.stdv[tid]; }
+  float* s_mean = par + DISC_MAX_PAR - 2 * KIN;
+  float* s_inv = s_mean + KIN;
+  if (tid < KIN) {
+    const bool in_ = IN == 0 || tid < nin;                            // padding columns: mean 0, 1 / std 0
+    s_mean[tid] = in_ ? a.mean[tid] : 0.f;
+    s_inv[tid] = in_ ? 1.0f / a.stdv[tid] : 0.f;
+  }
   if (tid == 0) {
     for (int s_ = 0; s_ < 2; ++s_) { mbar_init(a_full(s_), NPROD); mbar_init(a_free(s_), 1); }
     for (int s_ = 0; s_ < NSB; ++s_) { mbar_init(b_full(s_), 1); mbar_init(b_free(s_), 1); }
@@ -483,7 +508,8 @@ __global__ void __launch_bounds__(320, 1) disc_reward_pg2_kernel(DiscArgs a) {
       for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const float* img = a.image;
         for (int nb = 0; nb < NB1; ++nb) {
-          copy_chunk(img, 256);
+#pragma unroll
+          for (int ch = 0; ch < NCH; ++ch) copy_chunk(img, 256);
           for (int c = 0; c < 8; ++c) copy_chunk(img, N2);
         }
         if (VAIL)
@@ -521,7 +547,8 @@ __global__ void __launch_bounds__(320, 1) disc_reward_pg2_kernel(DiscArgs a) {
       };
       for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         for (int nb = 0; nb < NB1; ++nb) {
-          mma_chunk(256, D1_COL, true);
+#pragma unroll
+          for (int ch = 0; ch < NCH; ++ch) mma_chunk(256, D1_COL, ch == 0);
           for (int c = 0; c < 8; ++c) mma_chunk(N2, D2_COL, nb == 0 && c == 0);
         }
         if (VAIL)
@@ -548,23 +575,31 @@ __global__ void __launch_bounds__(320, 1) disc_reward_pg2_kernel(DiscArgs a) {
       asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(a_full(ga & 1)) : "memory");
       ++ga;
     };
-    auto load_row = [&](int tile_, float (&raw)[16]) {
+    // this thread's 16 columns of every input chunk: input 32 ch + 16 half + k at [ch][k]
+    auto load_row = [&](int tile_, float (&raw)[NCH][16]) {
       const int env_ = tile_ * TILE + row;
 #pragma unroll
-      for (int k = 0; k < 16; ++k) raw[k] = (tile_ < ntiles && env_ < a.n) ? a.s[(size_t)(16 * half + k) * a.ld + env_] : 0.f;
+      for (int j = 0; j < 16 * NCH; ++j) {
+        const int r = KC * (j / 16) + 16 * half + j % 16;
+        raw[j / 16][j % 16] = (tile_ < ntiles && env_ < a.n && (IN == 0 || r < nin)) ? a.s[(size_t)r * a.ld + env_] : 0.f;
+      }
     };
-    float xn[16];
+    float xn[NCH][16];
     load_row(blockIdx.x, xn);
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
       const int env = tile * TILE + row;
       const bool live = env < a.n;
-      float x[16];
+      float x[NCH][16];
 #pragma unroll
-      for (int k = 0; k < 16; ++k) x[k] = live ? (xn[k] - s_mean[16 * half + k]) * s_inv[16 * half + k] : 0.f;
+      for (int j = 0; j < 16 * NCH; ++j) {
+        const int r = KC * (j / 16) + 16 * half + j % 16;
+        x[j / 16][j % 16] = live ? (xn[j / 16][j % 16] - s_mean[r]) * s_inv[r] : 0.f;
+      }
       load_row(tile + gridDim.x, xn);
 #pragma unroll 1
       for (int nb = 0; nb < NB1; ++nb) {
-        put_half(x);                                                     // layer 1, column block nb
+        put_half(x[0]);                                                  // layer 1, column block nb
+        if constexpr (NCH == 2) put_half(x[1]);
 #pragma unroll 1
         for (int c = 0; c < 8; ++c) {                                    // layer 2, K-chunks fed by this block
           if (c == 0) wait_chunk(ga - 1);
@@ -1145,9 +1180,16 @@ __global__ void __launch_bounds__(192, 2) disc_vail3_kernel(DiscArgs a) {
 constexpr int V4_KC = 32, V4_NSB = 6, V4_NSA = 2;
 constexpr int V4_STAGE_B = 128 * V4_KC * 4 * 2;          // 32 KB: 128 rows x 32 K, hi + lo
 constexpr int V4_ACC1A = 0, V4_ACC1B = 128, V4_ACC2 = 256, V4_AR = 384;
-constexpr int V4_BCHUNKS = 2 + 8 + 8;
-constexpr int V4_ACHUNKS = 13;
 enum { V4_R1A = 0, V4_R1B, V4_R2, V4_R3A, V4_R3B, V4_NR };
+// With NCH input chunks a tile is NCH + 12 A chunks and 2 NCH + 16 B chunks (both layer-1 blocks read every input chunk).
+// The weight ring has as many stages as divide the B chunk count -- six for one input chunk (18 B chunks), five for two
+// (20) -- so that the stage of every chunk of the unrolled tile body is a compile-time constant.
+__host__ __device__ constexpr int v4_bchunks(int nch) { return 2 * nch + 16; }
+__host__ __device__ constexpr int v4_nsb(int nch) { return v4_bchunks(nch) % V4_NSB == 0 ? V4_NSB : 5; }
+__host__ __device__ constexpr size_t v4_smem(int nch) {
+  return (size_t)v4_nsb(nch) * V4_STAGE_B + (V2_NPAR + 3 + 2 * KC * nch + 256) * sizeof(float) +
+         (2 * V4_NSA + 2 * v4_nsb(nch) + V4_NR + 2) * 8 + 16;
+}
 
 //
 // Where the time goes (clock counters in the MMA-issuing thread and in a producer thread; experiments that are not in the
@@ -1178,16 +1220,20 @@ enum { V4_R1A = 0, V4_R1B, V4_R2, V4_R3A, V4_R3B, V4_NR };
 // 2 = the three accumulator blocks change roles from tile to tile instead, (L1a/L3a, L1b/L3b, L2)(i + 1) = (L2, L1a/L3a,
 // L1b/L3b)(i): the next tile's first layer-1 block goes into the block this tile's layer 2 used (read out once A12
 // exists), its second into the one head a has finished with, its layer 2 into the one head b has finished with.
-template <bool KL, int ROT>
-__global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
+template <bool KL, int ROT, int IN = 0>
+__global__ void __launch_bounds__(320, 1) disc_vail4_kernel(typename DiscInput<IN>::Args a) {
+  constexpr int NCH = DiscInput<IN>::NCH, KIN = KC * NCH;            // input chunks, padded input width
+  constexpr int NSB = v4_nsb(NCH), BCH = v4_bchunks(NCH), ACH = NCH + 12;
+  static_assert(IN == 0 || ROT == 0, "other input widths: the default schedule only");
+  const int nin = DiscInput<IN>::n_in(a);
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* ring = smem;
-  float* par = reinterpret_cast<float*>(smem + V4_NSB * V4_STAGE_B);
+  float* par = reinterpret_cast<float*>(smem + NSB * V4_STAGE_B);
   float* s_mean = par + V2_NPAR + 3;
-  float* s_inv = s_mean + DISC_IN;
-  float* red = s_inv + DISC_IN;                                 // [2][128] partial head sums of the second warpgroup
+  float* s_inv = s_mean + KIN;
+  float* red = s_inv + KIN;                                     // [2][128] partial head sums of the second warpgroup
   uint64_t* bars = reinterpret_cast<uint64_t*>(red + 256);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * V4_NSA + 2 * V4_NSB + V4_NR + 2);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * V4_NSA + 2 * NSB + V4_NR + 2);
   const float* b1 = par;
   const float* b2 = par + 256;
   const float* b3 = par + 384;            // per 128-row block h: [bmu[64h..64h+63], blv[64h..64h+63]]
@@ -1197,9 +1243,9 @@ __global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
   auto a_full = [&](int s_) { return bar0 + 8u * s_; };
   auto a_free = [&](int s_) { return bar0 + 8u * (V4_NSA + s_); };
   auto b_full = [&](int s_) { return bar0 + 8u * (2 * V4_NSA + s_); };
-  auto b_free = [&](int s_) { return bar0 + 8u * (2 * V4_NSA + V4_NSB + s_); };
-  auto ready = [&](int k) { return bar0 + 8u * (2 * V4_NSA + 2 * V4_NSB + k); };
-  const uint32_t h_done = bar0 + 8u * (2 * V4_NSA + 2 * V4_NSB + V4_NR);       // head b (and, without ROT, head a) has read
+  auto b_free = [&](int s_) { return bar0 + 8u * (2 * V4_NSA + NSB + s_); };
+  auto ready = [&](int k) { return bar0 + 8u * (2 * V4_NSA + 2 * NSB + k); };
+  const uint32_t h_done = bar0 + 8u * (2 * V4_NSA + 2 * NSB + V4_NR);          // head b (and, without ROT, head a) has read
   const uint32_t h_done_a = h_done + 8u;                                       // ROT: head a has read its block
   constexpr bool EARLY = ROT == 1 || ROT == 2;     // the next tile's input chunk is handed over before this tile's heads
   constexpr bool ALT = ROT == 3;                   // the two producer warpgroups take alternate A chunks (one ring stage each)
@@ -1214,7 +1260,8 @@ __global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
   // Prologue: the first weight chunks and the first input rows are requested BEFORE the parameter loads, the TMEM
   // allocation and the CTA-wide barrier, so that their DRAM / L2 latency runs under those (at 65536 samples a CTA has only
   // three or four tiles: every microsecond in front of the first MMA is 1.5 % of the call).
-  float xn[ALT ? 32 : 16];
+  // (16 NCH values: this thread's 16 columns of every input chunk, input 32 ch + 16 half + k at 16 ch + k)
+  float xn[ALT ? 32 : 16 * NCH];
   if (warp < 8) {
     const int half_ = warp >> 2;
     if (ALT) {                                      // warpgroup h hands over the input chunk of tiles h, h + 2, ...: whole rows
@@ -1224,15 +1271,20 @@ __global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
     } else {
       const int env_ = blockIdx.x * TILE + (tid & 127);
 #pragma unroll
-      for (int k = 0; k < 16; ++k) xn[k] = env_ < a.n ? a.s[(size_t)(16 * half_ + k) * a.ld + env_] : 0.f;
+      for (int ch = 0; ch < NCH; ++ch)
+#pragma unroll
+        for (int k = 0; k < 16; ++k) {
+          const int r = KC * ch + 16 * half_ + k;
+          xn[16 * ch + k] = (env_ < a.n && (IN == 0 || r < nin)) ? a.s[(size_t)r * a.ld + env_] : 0.f;
+        }
     }
   }
   int q_first = 0;                                                  // weight chunks already requested (copy thread only)
   if (tid == 288) {
-    for (int s_ = 0; s_ < V4_NSB; ++s_) { mbar_init(b_full(s_), 1); mbar_init(b_free(s_), 1); }
+    for (int s_ = 0; s_ < NSB; ++s_) { mbar_init(b_full(s_), 1); mbar_init(b_free(s_), 1); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    const int total = my_tiles * V4_BCHUNKS;
-    for (; q_first < V4_NSB && q_first < total; ++q_first) {
+    const int total = my_tiles * BCH;
+    for (; q_first < NSB && q_first < total; ++q_first) {
       mbar_expect_tx(b_full(q_first), V4_STAGE_B);
       const uint8_t* src = reinterpret_cast<const uint8_t*>(a.image) + (size_t)q_first * V4_STAGE_B;
       const uint32_t dst = smem_u32(ring + q_first * V4_STAGE_B);
@@ -1241,7 +1293,11 @@ __global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
     }
   }
   for (int i = tid; i < V2_NPAR; i += 320) par[i] = a.params[i];
-  if (tid < DISC_IN) { s_mean[tid] = a.mean[tid]; s_inv[tid] = 1.0f / a.stdv[tid]; }
+  if (tid < KIN) {
+    const bool in_ = IN == 0 || tid < nin;                            // padding columns: mean 0, 1 / std 0
+    s_mean[tid] = in_ ? a.mean[tid] : 0.f;
+    s_inv[tid] = in_ ? 1.0f / a.stdv[tid] : 0.f;
+  }
   if (tid == 0) {
     for (int s_ = 0; s_ < V4_NSA; ++s_) { mbar_init(a_full(s_), ALT ? 128 : 256); mbar_init(a_free(s_), 1); }
     for (int k = 0; k < V4_NR; ++k) mbar_init(ready(k), 1);
@@ -1256,14 +1312,14 @@ __global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
   const uint32_t tmem = *tmem_slot;
 
   if (warp == 9) {
-    // ===================================================== weight-copy issuer: 18 chunks of 32 KB per tile, MMA order
+    // ===================================================== weight-copy issuer: 18 (20) chunks of 32 KB per tile, MMA order
     if (tid == 288) {
-      const int total = my_tiles * V4_BCHUNKS;
+      const int total = my_tiles * BCH;
       for (int q = q_first; q < total; ++q) {
-        const int st = q % V4_NSB, use = q / V4_NSB;
+        const int st = q % NSB, use = q / NSB;
         if (use > 0) mbar_wait(b_free(st), (uint32_t)(use - 1) & 1u);
         mbar_expect_tx(b_full(st), V4_STAGE_B);
-        const uint8_t* src = reinterpret_cast<const uint8_t*>(a.image) + (size_t)(q % V4_BCHUNKS) * V4_STAGE_B;
+        const uint8_t* src = reinterpret_cast<const uint8_t*>(a.image) + (size_t)(q % BCH) * V4_STAGE_B;
         const uint32_t dst = smem_u32(ring + st * V4_STAGE_B);
 #pragma unroll
         for (int p = 0; p < 4; ++p) bulk_g2s(dst + p * (V4_STAGE_B / 4), src + p * (V4_STAGE_B / 4), V4_STAGE_B / 4, b_full(st));
@@ -1274,12 +1330,13 @@ __global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
     // One thread issues 216 MMAs per tile, and its own instruction stream is what paces them if it is not kept short: a
     // back-to-back M128 x N128 x K8 TF32 MMA takes 64 cycles (tools/micro/umma_rate.cu, SS and TS alike), but with the
     // stage index a run-time value every shared-memory descriptor cost four dependent uniform-datapath instructions and
-    // an MMA went out every 92 cycles.  18 weight chunks per tile is a multiple of the six stages, so with the tile body
-    // unrolled the stage of every chunk is a compile-time constant and a descriptor is ONE add: (ring address >> 4) +
-    // (constant offset | the constant leading-byte-offset field); the A chunks alternate between two TMEM stages whose
-    // order flips from tile to tile (13 chunks per tile), kept as two registers that are swapped.
+    // an MMA went out every 92 cycles.  18 weight chunks per tile is a multiple of the six stages (20 of the five with two
+    // input chunks), so with the tile body unrolled the stage of every chunk is a compile-time constant and a descriptor
+    // is ONE add: (ring address >> 4) + (constant offset | the constant leading-byte-offset field); the A chunks alternate
+    // between two TMEM stages whose order flips from tile to tile when a tile has an odd number of them (13 with one
+    // input chunk), kept as two registers that are swapped.
     if (elect_one_sync()) {
-      static_assert(V4_BCHUNKS % V4_NSB == 0 && V4_ACHUNKS % V4_NSA == 1, "stage bookkeeping of the unrolled tile body");
+      static_assert(BCH % NSB == 0, "stage bookkeeping of the unrolled tile body");
       const uint32_t idesc = idesc_tf32(TILE, 128);
       constexpr uint32_t LBO16 = 128, SBO16 = 8;                        // 2048 B and 128 B in 16-byte units
       constexpr uint32_t DESC_HI = SBO16 | (1u << 14);                  // bits 32..45 stride byte offset, bit 46 version 1
@@ -1290,14 +1347,15 @@ __global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
       int ga = 0;
       for (int it = 0; it < my_tiles; ++it) {
         const uint32_t P = tmem + acc_p(it), Q = tmem + acc_q(it), R = tmem + acc_r(it);
-        const uint32_t itp = (uint32_t)it & 1u;
-        // B chunk q of the tile (stage q % 6, its (3 it + q / 6)-th use) against the A chunk in TMEM stage `ab`:
+        // (parity of the uses of a weight stage before this tile: BCH / NSB uses per tile)
+        const uint32_t itp = (BCH / NSB) % 2 ? (uint32_t)it & 1u : 0u;
+        // B chunk q of the tile (stage q % NSB, its (BCH / NSB it + q / NSB)-th use) against the A chunk in TMEM stage `ab`:
         // 4 k-steps x (lo.hi, hi.lo, hi.hi)
         // (the weights are waited for BEFORE the A chunk: they arrive chunks ahead, the A chunk is what the MMA pipe is
         // waiting for, and every mbarrier wait costs the issuing thread ~100 cycles even when the phase is long complete)
-        auto wait_b = [&](int q) { mbar_wait(b_full(q % V4_NSB), (itp ^ (uint32_t)(q / V4_NSB)) & 1u); tc_fence_after(); };
+        auto wait_b = [&](int q) { mbar_wait(b_full(q % NSB), (itp ^ (uint32_t)(q / NSB)) & 1u); tc_fence_after(); };
         auto mma_chunk = [&](int q, uint32_t ab, uint32_t d, bool first) {
-          const int sb = q % V4_NSB;
+          const int sb = q % NSB;
 #pragma unroll
           for (int j = 0; j < V4_KC / 8; ++j) {
             const uint64_t dbh = bdesc((uint32_t)(sb * (V4_STAGE_B / 16) + j * 2 * LBO16));
@@ -1322,40 +1380,45 @@ __global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
         //        head a, R for head b.
         if ((ROT == 0 || ROT == 3) && it > 0) { mbar_wait(h_done, (uint32_t)(it - 1) & 1u); tc_fence_after(); }
         if (ROT == 1 && it > 0) { mbar_wait(h_done_a, (uint32_t)(it - 1) & 1u); tc_fence_after(); }
-        wait_b(0);
-        uint32_t ab = next_a(0);                                        // A0 = x
-        mma_chunk(0, ab, P, true);
-        umma_commit(ready(V4_R1A));
-        wait_b(1);
-        if (ROT == 2 && it > 0) { mbar_wait(h_done_a, (uint32_t)(it - 1) & 1u); tc_fence_after(); }
-        if (ROT == 1 && it > 0) { mbar_wait(h_done, (uint32_t)(it - 1) & 1u); tc_fence_after(); }
-        mma_chunk(1, ab, Q, true);
-        umma_commit(a_fr[0]);
+        uint32_t ab;
+#pragma unroll
+        for (int k = 0; k < NCH; ++k) {                                 // A0 (A0, A1) = x -> layer-1 blocks a and b
+          wait_b(2 * k);
+          ab = next_a(k);
+          mma_chunk(2 * k, ab, P, k == 0);
+          if (k == NCH - 1) umma_commit(ready(V4_R1A));
+          wait_b(2 * k + 1);
+          if (ROT == 2 && it > 0) { mbar_wait(h_done_a, (uint32_t)(it - 1) & 1u); tc_fence_after(); }
+          if (ROT == 1 && it > 0) { mbar_wait(h_done, (uint32_t)(it - 1) & 1u); tc_fence_after(); }
+          mma_chunk(2 * k + 1, ab, Q, k == 0);
+          umma_commit(a_fr[k & 1]);
+        }
         umma_commit(ready(V4_R1B));
         if (ROT == 2 && it > 0) { mbar_wait(h_done, (uint32_t)(it - 1) & 1u); tc_fence_after(); }
 #pragma unroll
-        for (int c = 0; c < 8; ++c) {                                   // A1..A8 -> layer 2
-          wait_b(2 + c);
-          ab = next_a(1 + c);
-          mma_chunk(2 + c, ab, R, c == 0);
-          umma_commit(a_fr[(1 + c) & 1]);
+        for (int c = 0; c < 8; ++c) {                                   // A1..A8 (A2..A9) -> layer 2
+          wait_b(2 * NCH + c);
+          ab = next_a(NCH + c);
+          mma_chunk(2 * NCH + c, ab, R, c == 0);
+          umma_commit(a_fr[(NCH + c) & 1]);
         }
         umma_commit(ready(V4_R2));
 #pragma unroll
-        for (int c = 0; c < 4; ++c) {                                   // A9..A12 -> [mu; lv] blocks a and b
-          wait_b(10 + 2 * c);
-          ab = next_a(9 + c);
-          mma_chunk(10 + 2 * c, ab, P, c == 0);
+        for (int c = 0; c < 4; ++c) {                                   // A9..A12 (A10..A13) -> [mu; lv] blocks a and b
+          wait_b(2 * NCH + 8 + 2 * c);
+          ab = next_a(NCH + 8 + c);
+          mma_chunk(2 * NCH + 8 + 2 * c, ab, P, c == 0);
           if (c == 3) umma_commit(ready(V4_R3A));
-          wait_b(11 + 2 * c);
-          mma_chunk(11 + 2 * c, ab, Q, c == 0);
-          umma_commit(a_fr[(9 + c) & 1]);
+          wait_b(2 * NCH + 9 + 2 * c);
+          mma_chunk(2 * NCH + 9 + 2 * c, ab, Q, c == 0);
+          umma_commit(a_fr[(NCH + 8 + c) & 1]);
         }
         umma_commit(ready(V4_R3B));
-        // 13 A chunks per tile: the next tile's even chunks live in the other stage
-        { const uint32_t t_ = a_st[0]; a_st[0] = a_st[1]; a_st[1] = t_; }
-        { const uint32_t t_ = a_fu[0]; a_fu[0] = a_fu[1]; a_fu[1] = t_; }
-        { const uint32_t t_ = a_fr[0]; a_fr[0] = a_fr[1]; a_fr[1] = t_; }
+        if constexpr (ACH % V4_NSA == 1) {                              // the next tile's even chunks live in the other stage
+          { const uint32_t t_ = a_st[0]; a_st[0] = a_st[1]; a_st[1] = t_; }
+          { const uint32_t t_ = a_fu[0]; a_fu[0] = a_fu[1]; a_fu[1] = t_; }
+          { const uint32_t t_ = a_fr[0]; a_fr[0] = a_fr[1]; a_fr[1] = t_; }
+        }
       }
     }
   } else {
@@ -1410,17 +1473,28 @@ __global__ void __launch_bounds__(320, 1) disc_vail4_kernel(DiscArgs a) {
       }
     };
     auto wait_ready = [&](int k, int it) { mbar_wait(ready(k), (uint32_t)it & 1u); tc_fence_after(); };
-    auto load_row = [&](int tile_, float (&raw)[16]) {
+    auto load_row = [&](int tile_, float (&raw)[16 * NCH]) {
       const int env_ = tile_ * TILE + row;
 #pragma unroll
-      for (int k = 0; k < 16; ++k) raw[k] = (tile_ < ntiles && env_ < a.n) ? a.s[(size_t)(16 * half + k) * a.ld + env_] : 0.f;
-    };
-    auto put_input = [&](int tile_) {                                   // A0 of tile_ from the prefetched row
-      const bool live_ = tile_ * TILE + row < a.n;
-      float x[16];
+      for (int ch = 0; ch < NCH; ++ch)
 #pragma unroll
-      for (int k = 0; k < 16; ++k) x[k] = live_ ? (xn[k] - s_mean[16 * half + k]) * s_inv[16 * half + k] : 0.f;
-      put(x);
+        for (int k = 0; k < 16; ++k) {
+          const int r = KC * ch + 16 * half + k;
+          raw[16 * ch + k] = (tile_ < ntiles && env_ < a.n && (IN == 0 || r < nin)) ? a.s[(size_t)r * a.ld + env_] : 0.f;
+        }
+    };
+    auto put_input = [&](int tile_) {                                   // A0 (A0, A1) of tile_ from the prefetched row
+      const bool live_ = tile_ * TILE + row < a.n;
+#pragma unroll
+      for (int ch = 0; ch < NCH; ++ch) {
+        float x[16];
+#pragma unroll
+        for (int k = 0; k < 16; ++k) {
+          const int r = KC * ch + 16 * half + k;
+          x[k] = live_ ? (xn[16 * ch + k] - s_mean[r]) * s_inv[r] : 0.f;
+        }
+        put(x);
+      }
     };
     int it = 0;
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++it) {
@@ -1554,6 +1628,7 @@ using namespace om;
 
 struct OmDisc {
   DiscShape sh;
+  int n_in;                     // 32: every kernel; otherwise the default kernels only (image4 + params2 / image + params)
   float* image = nullptr;
   float* params = nullptr;
   float* image2 = nullptr;      // VAIL: chunk image / parameters of disc_vail2_kernel
@@ -1589,20 +1664,28 @@ static void append_chunk(std::vector<float>& img, const float* w, int ldw, int r
 
 extern "C" int om_disc_create(const OmDiscDesc* d, OmDisc** out) {
   OM_REQUIRE(d && out, "om_disc_create: null argument");
-  OM_REQUIRE(d->n_in == DISC_IN, "om_disc_create: n_in must be %d (the H1 observation), got %d", DISC_IN, d->n_in);
+  OM_REQUIRE(d->n_in >= 1 && d->n_in <= DISC_MAX_IN, "om_disc_create: n_in must be 1..%d, got %d", DISC_MAX_IN, d->n_in);
   const bool vail = d->kind == 0;
   OM_REQUIRE(d->kind == 0 || d->kind == 1, "om_disc_create: kind must be 0 (VAIL) or 1 (GAIL)");
   OM_REQUIRE((vail && d->n_h1 == 256 && d->n_h2 == 128 && d->z_size == 128) || (!vail && d->n_h1 == 512 && d->n_h2 == 256),
-             "om_disc_create: only the reference shapes are built (VAIL 32-256-128-z128-1, GAIL 32-512-256-1)");
+             "om_disc_create: only the reference shapes are built (VAIL n_in-256-128-z128-1, GAIL n_in-512-256-1)");
   OM_REQUIRE(d->w1 && d->b1 && d->w2 && d->b2 && d->wd && d->bd, "om_disc_create: null weights");
   OM_REQUIRE(!vail || (d->wmu && d->bmu && d->wlv && d->blv), "om_disc_create: VAIL needs mu / logvar layers");
   const int n1 = d->n_h1, n2 = d->n_h2, z = vail ? d->z_size : 0;
+  // W1 in whole 32-column input chunks, the padding columns zero.  The earlier kernels, reachable through the
+  // disc_vail2 / disc_pg2 knobs only, take 32 inputs: their images are built for that width alone.
+  const int n_in = d->n_in, nch = ceil_div(n_in, KC), kin = KC * nch;
+  const bool all_kernels = n_in == DISC_IN;
+  std::vector<float> w1((size_t)n1 * kin, 0.f);
+  for (int r = 0; r < n1; ++r) std::memcpy(&w1[(size_t)r * kin], d->w1 + (size_t)r * n_in, sizeof(float) * n_in);
   std::vector<float> img;
-  for (int nb = 0; nb < n1 / 256; ++nb) {
-    append_chunk(img, d->w1, DISC_IN, nb * 256, 256, 0);
-    for (int c = 0; c < 8; ++c) append_chunk(img, d->w2, n1, 0, n2, nb * 256 + c * KC);
+  if (!vail || all_kernels) {
+    for (int nb = 0; nb < n1 / 256; ++nb) {
+      for (int ch = 0; ch < nch; ++ch) append_chunk(img, w1.data(), kin, nb * 256, 256, ch * KC);
+      for (int c = 0; c < 8; ++c) append_chunk(img, d->w2, n1, 0, n2, nb * 256 + c * KC);
+    }
   }
-  if (vail) {
+  if (vail && all_kernels) {
     std::vector<float> w3((size_t)2 * z * n2);                 // [mu; logvar] stacked: 2z rows x n2
     std::memcpy(w3.data(), d->wmu, sizeof(float) * z * n2);
     std::memcpy(w3.data() + (size_t)z * n2, d->wlv, sizeof(float) * z * n2);
@@ -1639,12 +1722,14 @@ extern "C" int om_disc_create(const OmDiscDesc* d, OmDisc** out) {
             split_tf32(w[(size_t)(r0 + r) * ldw + k0 + kc * 4 + e], hi + ((size_t)kc * V2_ROWS + r) * 4 + e,
                        lo + ((size_t)kc * V2_ROWS + r) * 4 + e);
     };
-    for (int blk = 0; blk < 2; ++blk) {
-      for (int c = 0; c < 2; ++c) chunk16(d->w1, DISC_IN, 128 * blk, 16 * c);
-      for (int c = 0; c < 8; ++c) chunk16(d->w2, n1, 0, 128 * blk + 16 * c);
+    if (all_kernels) {
+      for (int blk = 0; blk < 2; ++blk) {
+        for (int c = 0; c < 2; ++c) chunk16(d->w1, DISC_IN, 128 * blk, 16 * c);
+        for (int c = 0; c < 8; ++c) chunk16(d->w2, n1, 0, 128 * blk + 16 * c);
+      }
+      for (int hb = 0; hb < 2; ++hb)
+        for (int c = 0; c < 8; ++c) chunk16(w3i.data(), n2, 128 * hb, 16 * c);
     }
-    for (int hb = 0; hb < 2; ++hb)
-      for (int c = 0; c < 8; ++c) chunk16(w3i.data(), n2, 128 * hb, 16 * c);
     par2.insert(par2.end(), d->b1, d->b1 + n1);
     par2.insert(par2.end(), d->b2, d->b2 + n2);
     par2.insert(par2.end(), b3i.begin(), b3i.end());
@@ -1654,7 +1739,7 @@ extern "C" int om_disc_create(const OmDiscDesc* d, OmDisc** out) {
   // ---- VAIL with the A operand in TMEM (disc_vail3_kernel): 64-row blocks of layer 1 and of [mu; logvar] (rows
   //      interleaved per 32), 128-row chunks of layer 2, all 16 columns wide, in the kernel's issue order
   std::vector<float> img3, par3;
-  if (vail) {
+  if (vail && all_kernels) {
     std::vector<float> w3i((size_t)2 * z * n2), b3i(2 * z);
     for (int hb = 0; hb < 4; ++hb)
       for (int r = 0; r < 32; ++r) {
@@ -1687,8 +1772,8 @@ extern "C" int om_disc_create(const OmDiscDesc* d, OmDisc** out) {
     par3.insert(par3.end(), d->wd, d->wd + z);
     par3.push_back(d->bd[0]);
   }
-  // ---- VAIL, one CTA per SM, A operand in TMEM (disc_vail4_kernel): 18 chunks of 128 rows x 32 columns in MMA order;
-  //      the [mu; logvar] rows interleaved per 64 exactly as for disc_vail2_kernel (whose parameter block it shares)
+  // ---- VAIL, one CTA per SM, A operand in TMEM (disc_vail4_kernel): 2 nch + 16 chunks of 128 rows x 32 columns in MMA
+  //      order; the [mu; logvar] rows interleaved per 64 exactly as for disc_vail2_kernel (whose parameter block it shares)
   std::vector<float> img4;
   if (vail) {
     std::vector<float> w3i((size_t)2 * z * n2);
@@ -1708,8 +1793,10 @@ extern "C" int om_disc_create(const OmDiscDesc* d, OmDisc** out) {
             split_tf32(w[(size_t)(r0 + r) * ldw + k0 + kc * 4 + e], hi + ((size_t)kc * 128 + r) * 4 + e,
                        lo + ((size_t)kc * 128 + r) * 4 + e);
     };
-    chunk32(d->w1, DISC_IN, 0, 0);
-    chunk32(d->w1, DISC_IN, 128, 0);
+    for (int ch = 0; ch < nch; ++ch) {
+      chunk32(w1.data(), kin, 0, KC * ch);
+      chunk32(w1.data(), kin, 128, KC * ch);
+    }
     for (int c = 0; c < 8; ++c) chunk32(d->w2, n1, 0, 32 * c);
     for (int c = 0; c < 4; ++c) {
       chunk32(w3i.data(), n2, 0, 32 * c);
@@ -1718,22 +1805,19 @@ extern "C" int om_disc_create(const OmDiscDesc* d, OmDisc** out) {
   }
   OmDisc* h = new OmDisc();
   h->sh = DiscShape{d->kind, n1, n2, z};
-  cudaError_t e = cudaMalloc(&h->image, img.size() * sizeof(float));
-  if (e == cudaSuccess) e = cudaMalloc(&h->params, par.size() * sizeof(float));
-  if (e == cudaSuccess) e = cudaMemcpy(h->image, img.data(), img.size() * sizeof(float), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(h->params, par.data(), par.size() * sizeof(float), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess && vail) {
-    e = cudaMalloc(&h->image2, img2.size() * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&h->params2, par2.size() * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemcpy(h->image2, img2.data(), img2.size() * sizeof(float), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(h->params2, par2.data(), par2.size() * sizeof(float), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMalloc(&h->image3, img3.size() * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&h->params3, par3.size() * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemcpy(h->image3, img3.data(), img3.size() * sizeof(float), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(h->params3, par3.data(), par3.size() * sizeof(float), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMalloc(&h->image4, img4.size() * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemcpy(h->image4, img4.data(), img4.size() * sizeof(float), cudaMemcpyHostToDevice);
-  }
+  h->n_in = n_in;
+  cudaError_t e = cudaSuccess;
+  auto upload = [&](const std::vector<float>& v, float** dst) {           // an image not built stays null
+    if (e == cudaSuccess && !v.empty()) e = cudaMalloc(dst, v.size() * sizeof(float));
+    if (e == cudaSuccess && !v.empty()) e = cudaMemcpy(*dst, v.data(), v.size() * sizeof(float), cudaMemcpyHostToDevice);
+  };
+  upload(img, &h->image);
+  upload(par, &h->params);
+  upload(img2, &h->image2);
+  upload(par2, &h->params2);
+  upload(img3, &h->image3);
+  upload(par3, &h->params3);
+  upload(img4, &h->image4);
   if (e != cudaSuccess) {
     if (h->image) cudaFree(h->image);
     if (h->params) cudaFree(h->params);
@@ -1751,7 +1835,7 @@ extern "C" int om_disc_create(const OmDiscDesc* d, OmDisc** out) {
 
 extern "C" void om_disc_destroy(OmDisc* h) {
   if (!h) return;
-  cudaFree(h->image);
+  if (h->image) cudaFree(h->image);
   cudaFree(h->params);
   if (h->image2) cudaFree(h->image2);
   if (h->params2) cudaFree(h->params2);
@@ -1782,6 +1866,32 @@ extern "C" int om_disc_forward(const OmDisc* h, const float* s, const float* mea
   const size_t smem = 2 * STAGE_A_BYTES + NSB * STAGE_B2_BYTES + (DISC_MAX_PAR + 4) * sizeof(float) + 12 * 8 + 16;
   DiscArgs a{h->sh, h->image, h->params, s, mean, stdv, eps, reward, d_out, kl_out, n, ld};
   cudaStream_t st = (cudaStream_t)stream;
+  if (h->n_in != DISC_IN) {
+    // another input width: the default kernels, built for one or two input chunks
+    const bool knob = h->sh.kind == 0 ? !(g_knobs.disc_vail2 < 0 || g_knobs.disc_vail2 == 4) : g_knobs.disc_pg2 == 0;
+    OM_REQUIRE(!knob, "om_disc_forward: the kernel variant the disc_vail2 / disc_pg2 knob selects takes %d inputs only, "
+               "this network has %d", DISC_IN, h->n_in);
+    DiscArgsIn aw;
+    static_cast<DiscArgs&>(aw) = a;
+    aw.n_in = h->n_in;
+    const bool two_ch = h->n_in > KC;
+    if (h->sh.kind == 0) {
+      aw.image = h->image4;
+      aw.params = h->params2;
+      const size_t smem4 = v4_smem(two_ch ? 2 : 1);
+      auto kern = two_ch ? (kl_out ? disc_vail4_kernel<true, 0, 2> : disc_vail4_kernel<false, 0, 2>)
+                         : (kl_out ? disc_vail4_kernel<true, 0, 1> : disc_vail4_kernel<false, 0, 1>);
+      OM_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4));
+      kern<<<grid, 320, smem4, st>>>(aw);
+    } else {
+      const size_t smem_pg2 = smem + 2 * 128 * sizeof(float);         // the standardiser slots lie inside DISC_MAX_PAR
+      auto kern = two_ch ? disc_reward_pg2_kernel<512, 256, false, false, 2> : disc_reward_pg2_kernel<512, 256, false, false, 1>;
+      OM_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pg2));
+      kern<<<grid, 320, smem_pg2, st>>>(aw);
+    }
+    OM_LAUNCHED();
+    return 0;
+  }
   // VAIL: two CTAs per SM.  (The two-producer-group kernel below is 3 % faster at 65536 samples when timed alone -- 73.4
   // vs 76.3 us -- but 15 % slower inside bench.py's process, after the large-buffer measurements: 88.8 us; the two-CTA
   // kernel reads 76-78 us in both settings, so it stays the default.)
@@ -1792,8 +1902,7 @@ extern "C" int om_disc_forward(const OmDisc* h, const float* s, const float* mea
   // two-producer-group shared-memory kernel (knob 0)
   if (h->sh.kind == 0 && (g_knobs.disc_vail2 == 4 || g_knobs.disc_vail2 == 5 || g_knobs.disc_vail2 == 6 || g_knobs.disc_vail2 == 7 ||
                             g_knobs.disc_vail2 < 0)) {
-    const size_t smem4 = V4_NSB * V4_STAGE_B + (V2_NPAR + 3 + 2 * DISC_IN + 256) * sizeof(float) +
-                         (2 * V4_NSA + 2 * V4_NSB + V4_NR + 2) * 8 + 16;
+    const size_t smem4 = v4_smem(1);
     const int rot = g_knobs.disc_vail2 == 5 ? 2 : g_knobs.disc_vail2 == 6 ? 1 : g_knobs.disc_vail2 == 7 ? 3 : 0;
     DiscArgs a4 = a;
     a4.image = h->image4;

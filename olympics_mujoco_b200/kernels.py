@@ -484,8 +484,11 @@ def ppo_loss_stats(logp, old_logp, adv, clip, mask=None, values=None, returns=No
 # ------------------------------------------------------------------------------------------- discriminator (K4)
 class Discriminator:
     """OmDisc handle.  ``params``: dict of float32 arrays in torch.nn.Linear layout ([out, in] weights):
-    VAIL  w1 b1 w2 b2 wmu bmu wlv blv wd bd   (32-256-128-z128-1)
-    GAIL  w1 b1 w2 b2 w3 b3                   (32-512-256-1)"""
+    VAIL  w1 b1 w2 b2 wmu bmu wlv blv wd bd   (n_in-256-128-z128-1)
+    GAIL  w1 b1 w2 b2 w3 b3                   (n_in-512-256-1)
+    ``n_in`` (the columns of w1) is 1..64: the kinematic observation of any UnitreeH1 variant,
+    ``env.get_kinematic_obs_mask()`` (32 for the default model, 30 without the back joint, 48 with arms, 46 with arms
+    and without the back joint)."""
 
     def __init__(self, kind, params):
         _lib.require_cuda()
@@ -515,10 +518,11 @@ class Discriminator:
             pass
 
     def reward(self, s, mean, std, eps=None, want_d=False):
-        """s [32, n] observations (SoA), mean / std [32] float32 device tensors, eps [z, n] or None -> reward [n]
+        """s [n_in, n] observations (SoA), mean / std [n_in] float32 device tensors, eps [z, n] or None -> reward [n]
         (and the raw logit d [n] when ``want_d``)."""
         n = s.shape[-1]
         assert s.shape == (self.n_in, n) and (eps is None or eps.shape == (self.z, n))
+        assert mean.numel() == self.n_in and std.numel() == self.n_in
         reward = torch.empty(n, device=s.device)
         d = torch.empty(n, device=s.device) if want_d else None
         check(_lib.load().om_disc_reward(self.handle, _p(s, torch.float32), _p(mean, torch.float32), _p(std, torch.float32),
@@ -528,9 +532,10 @@ class Discriminator:
 
     def forward(self, s, mean, std, eps=None, want_reward=False, want_kl=None):
         """The forward pass of the discriminator FIT (gail_TRPO.py:167-220): -> dict(logit [n], kl [n] (VAIL),
-        reward [n] if asked).  Same kernel as ``reward``; the KL term is VDBLoss.kl_divergence per sample."""
+        reward [n] if asked) for s [n_in, n].  Same kernel as ``reward``; the KL term is VDBLoss.kl_divergence per sample."""
         n = s.shape[-1]
         assert s.shape == (self.n_in, n) and (eps is None or eps.shape == (self.z, n))
+        assert mean.numel() == self.n_in and std.numel() == self.n_in
         want_kl = (self.kind == 0) if want_kl is None else want_kl
         out = dict(logit=torch.empty(n, device=s.device))
         if want_kl:

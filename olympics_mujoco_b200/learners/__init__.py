@@ -46,7 +46,9 @@ def normalize_advantage_ppo(adv, eps=1e-5):
 
 class DiscriminatorReward:
     """The reward side of GAIL / VAIL for the UnitreeH1 configuration (state-only discriminator,
-    ``use_next_states=False, use_actions=False``; ``examples/imitation_learning/utils.py:151-179``)."""
+    ``use_next_states=False, use_actions=False``; ``examples/imitation_learning/utils.py:151-179``).  The input width
+    n_in is that of ``params["w1"]``: the kinematic observation of the env's variant, ``env.get_kinematic_obs_mask()``
+    (1..64 inputs)."""
 
     def __init__(self, kind, params, device="cuda", seed=0):
         self.kind = kind.lower()
@@ -55,7 +57,7 @@ class DiscriminatorReward:
         self._gen = torch.Generator(device=device).manual_seed(seed)
 
     def make_discrim_reward(self, state, action=None, next_state=None, eps=None, update_standardizer=True):
-        """state [32, n] (SoA) -> reward [n] float32.  Like the reference, every call first folds the batch into the
+        """state [n_in, n] (SoA) -> reward [n] float32.  Like the reference, every call first folds the batch into the
         standardiser's running sums (all ranks), then standardises with the updated statistics."""
         if update_standardizer:
             self.standardizer.update(state)
@@ -136,7 +138,8 @@ class VDBLoss(GailDiscriminatorLoss):
 def _fit_batch(self, plcy_state, expert, loss, eps=None, noisy_targets=False, logging_forwards=False):
     """One epoch of ``GAIL._fit_discriminator`` up to (not including) the weight update: sample the expert half, fold
     [policy; expert] into the standardiser, forward, loss + statistics.
-    -> (loss value, stats, batch dict with ``inputs`` [32, 2n], ``logit``, ``kl``, ``dlogit``, ``target``).
+    ``plcy_state`` [n_in, n]; ``expert`` an ExpertDataset masked to the same n_in columns.
+    -> (loss value, stats, batch dict with ``inputs`` [n_in, 2n], ``logit``, ``kl``, ``dlogit``, ``target``).
 
     Standardiser bookkeeping, as the reference does it: the discriminator's input standardiser and ``_D_standardizer``
     are ONE object (``examples/imitation_learning/utils.py``), and it updates on EVERY forward (``networks.py:66-71``).
@@ -146,6 +149,7 @@ def _fit_batch(self, plcy_state, expert, loss, eps=None, noisy_targets=False, lo
     each half: four batch-equivalents).  The same counts are replayed here (``logging_forwards`` = a writer is attached);
     the moment sums of a batch are computed once and added with the multiplicity."""
     n = plcy_state.shape[-1]
+    assert plcy_state.shape[0] == self.disc.n_in and expert.table.shape[0] == self.disc.n_in
     demo, _, _ = expert.sample(n)
     inputs = torch.cat([plcy_state, demo], dim=1)
     batch_moments = Kn.moments(inputs)

@@ -1,5 +1,9 @@
 """Timing of BASELINE.json configs[3]: VAIL / GAIL discriminator-reward rollout, 65536 envs (tcgen05 MLP).
-Prints one JSON line per network (measurement aid; the driver-facing bench is bench.py)."""
+Prints one JSON line per network (measurement aid; the driver-facing bench is bench.py).
+
+``--n-in 32 30 48 --rounds 3`` times the networks at other input widths (the UnitreeH1 variants' kinematic
+observations) in one process, alternating the widths round by round; a width other than 32 takes the reference weights
+with a seeded first layer of that width."""
 import argparse
 import json
 import sys
@@ -10,7 +14,12 @@ import torch
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
-FLOP = {"vail": 2 * (32 * 256 + 256 * 128 + 2 * 128 * 128 + 128), "gail": 2 * (32 * 512 + 512 * 256 + 256)}
+
+
+def flop(kind, n_in=32):
+    """Useful FLOP per sample, the first layer at the width the kernels compute: n_in rounded up to 32."""
+    k = 32 * -(-n_in // 32)
+    return {"vail": 2 * (k * 256 + 256 * 128 + 2 * 128 * 128 + 128), "gail": 2 * (k * 512 + 512 * 256 + 256)}[kind]
 
 
 _TF32_PEAK = None
@@ -45,22 +54,26 @@ def tf32_peak():
     return _TF32_PEAK
 
 
-def measure(envs=65536, steps=50, warmup=5):
+def measure(envs=65536, steps=50, warmup=5, n_in=32):
     args = argparse.Namespace(envs=envs, steps=steps, warmup=warmup)
     res = []
     from olympics_mujoco_b200 import kernels as Kn
     g = np.load(ROOT / "tests/golden/discriminator_ref.npz")
     n = args.envs
     gen = torch.Generator(device="cuda").manual_seed(0)
-    s = torch.randn((32, n), device="cuda", generator=gen)
+    s = torch.randn((n_in, n), device="cuda", generator=gen)
     eps = torch.randn((128, n), device="cuda", generator=gen)
-    mean, std = torch.zeros(32, device="cuda"), torch.ones(32, device="cuda")
+    mean, std = torch.zeros(n_in, device="cuda"), torch.ones(n_in, device="cuda")
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
     peaks = json.loads((ROOT / "MEASURED_PEAKS.json").read_text()) if (ROOT / "MEASURED_PEAKS.json").exists() else {"bf16_tflops": 1590.0}
     for kind in ("vail", "gail"):
         pref = "v_" if kind == "vail" else "g_"
         names = ("w1", "b1", "w2", "b2", "wmu", "bmu", "wlv", "blv", "wd", "bd") if kind == "vail" else ("w1", "b1", "w2", "b2", "w3", "b3")
-        disc = Kn.Discriminator(kind, {k: g[pref + k] for k in names})
+        params = {k: g[pref + k] for k in names}
+        if n_in != 32:
+            rng = np.random.default_rng(n_in)
+            params["w1"] = (rng.uniform(-1, 1, (params["w1"].shape[0], n_in)) / np.sqrt(n_in)).astype(np.float32)
+        disc = Kn.Discriminator(kind, params)
         e = eps if kind == "vail" else None
         for _ in range(args.warmup):
             disc.reward(s, mean, std, eps=e)
@@ -75,15 +88,18 @@ def measure(envs=65536, steps=50, warmup=5):
             torch.cuda.synchronize()
             tot += t0.elapsed_time(t1)
         ms = tot / args.steps
-        useful = FLOP[kind] * n / (ms * 1e-3) / 1e12
+        useful = flop(kind, n_in) * n / (ms * 1e-3) / 1e12
         peak_tf32 = tf32_peak()
-        res.append({"workload": f"{kind.upper()} discriminator reward, {n} envs (configs[3])", "net": kind, "ms": ms,
+        width = "" if n_in == 32 else f", {n_in} inputs"
+        res.append({"workload": f"{kind.upper()} discriminator reward, {n} envs{width} (configs[3])", "net": kind, "ms": ms,
                     "value": n / (ms * 1e-3), "unit": "samples/s",
                     "roofline": {"bound": "tensor", "achieved": useful, "executed_3xtf32": 3 * useful, "unit": "TFLOP/s",
                                  "peak": peak_tf32, "peak_note": "TF32 matmul 8192^3 measured in this process (best of 10)",
                                  "bf16_burst_half": peaks["bf16_tflops"] / 2,
                                  "frac": useful / peak_tf32, "frac_executed": 3 * useful / peak_tf32,
-                                 "flop_per_sample": FLOP[kind]}})
+                                 "flop_per_sample": flop(kind, n_in)}})
+        if n_in != 32:
+            res[-1]["n_in"] = n_in
     return res
 
 
@@ -92,9 +108,13 @@ def main():
     ap.add_argument("--envs", type=int, default=65536)
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--n-in", type=int, nargs="+", default=[32], help="input widths (1..64), timed in this order")
+    ap.add_argument("--rounds", type=int, default=1, help="repeat the sequence of widths, alternating them")
     a = ap.parse_args()
-    for r in measure(a.envs, a.steps, a.warmup):
-        print(json.dumps(r))
+    for _ in range(a.rounds):
+        for n_in in a.n_in:
+            for r in measure(a.envs, a.steps, a.warmup, n_in):
+                print(json.dumps(r))
 
 
 if __name__ == "__main__":
