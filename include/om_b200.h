@@ -234,6 +234,44 @@ int om_h1_live_step(const OmModel* m, const OmH1Spec* spec, const OmTraj* t, uin
 int om_h1_draw_models(uint64_t seed, uint32_t env_id0, uint32_t count, int n_models, int random,
                       const double* body_mass_host, int32_t* idx, float* mass, int n, void* stream);
 
+/* Per-env reset of a UnitreeH1 batch: LocoEnvBase.reset (loco_env_base.py:568-604, setup :606-657) for a subset of the envs,
+ * and mushroom_rl Core's reset on `last` (Core._step / _reset: last = absorbing or episode_steps >= horizon, then reset that
+ * env alone).  For every env that resets:
+ *   qpos = qpos0 of the model, qvel = 0 (mj_resetData); grf rows = 0 (mean_grf.reset(), :584);
+ *   trajectory reset under the om_traj_reset contract (key seed, counter (env_id0 + i, reset_count[i], 0, 0); reset_count[i]
+ *   += 1; forced_traj / forced_step >= 0 override the draw, as reset_trajectory(substep_no, traj_no) does);
+ *   set_sim_state of the drawn sample (root x, y re-centred to 0); obs = its observation (sample keys 2..K-1, then grf = 0);
+ *   prev_x_vel[i] = obs row spec->x_vel_idx; episode_step[i] = 0;
+ *   with model_index: the env draws its own model (see below).
+ * Modes:
+ *   mask != NULL  (explicit): env i resets iff mask[i] != 0; nothing of another env is written except its obs row (below).
+ *   mask == NULL  (auto-reset, after a step): episode_step[i] += 1, last[i] = absorbing[i] || episode_step[i] >= horizon,
+ *                 env i resets iff last[i]; prev_x_vel[i] = obs row x_vel_idx for EVERY env.  absorbing, episode_step, last,
+ *                 obs_in, obs and prev_x_vel are required.
+ * obs (may be NULL in explicit mode) [obs_dim][ld] = the observation after the call: the new one for envs that reset, row i of
+ * obs_in for the others (obs_in NULL: those rows are left alone; obs_in may equal obs).  obs_dim = 2 n_obs_q - 2 + n_grf.
+ * Model draw (model_index != NULL; the per-env carried weight): env i's j-th partial reset, j = partial_resets[i] (then
+ * incremented), takes model  random != 0: Philox(key seed; counter env_id0 + i, j, 33, 0) word 0 times n_models, high
+ * 32 bits;  random == 0: (model_index[i] + 1) mod n_models;  and mass[i] = masses_host[model_index[i]].
+ * qpos [nq][ld], qvel [nv][ld] of the model; the trajectory must have 2 n_obs_q keys.  No FK: the MjData mirrors (xpos ...)
+ * are not written.  Every call only enqueues one kernel (no allocation, no host synchronisation): capturable in a CUDA graph
+ * behind om_h1_step. */
+typedef struct OmH1ResetArgs {
+  const uint8_t* mask;                       /* [ld] explicit mode, or NULL = auto-reset mode */
+  const uint8_t* absorbing; int horizon;     /* auto-reset mode: the step's absorbing flags [ld], info.horizon */
+  int forced_traj, forced_step;              /* -1 = draw */
+  int32_t* traj_no; int32_t* step_no; uint32_t* reset_count; double* xy_off;   /* the OmTraj state ([ld], xy_off [2][ld]) */
+  float* qpos; float* qvel;
+  const float* obs_in; float* obs; int obs_dim;
+  float* prev_x_vel; int32_t* episode_step; uint8_t* last;   /* [ld]; episode_step may be NULL in explicit mode */
+  float* grf; int n_grf;                     /* [n_grf][ld] or NULL */
+  int32_t* partial_resets; int32_t* model_index; float* mass;   /* [ld] or all NULL */
+  int n_models, random;
+  const double* masses_host;                 /* [n_models] <= 16 */
+} OmH1ResetArgs;
+int om_h1_reset_envs(const OmModel* m, const OmH1Spec* spec, const OmTraj* t, uint64_t seed, uint32_t env_id0,
+                     const OmH1ResetArgs* args, int n, int ld, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * K2 (A3 flavour): the tail of StickFigureA3.step (real_humanoid_robots/StickFigureA3.py:187-202) after
  * robot.step (= mj_step, which stays the reference's): WalkingTask.step (tasks/walking_task.py:246-293),

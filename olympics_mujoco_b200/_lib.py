@@ -53,6 +53,16 @@ class OmLiveOut(C.Structure):
                                           "absorbing", "wrapped")]
 
 
+class OmH1ResetArgs(C.Structure):
+    _fields_ = [("mask", C.c_void_p), ("absorbing", C.c_void_p), ("horizon", C.c_int), ("forced_traj", C.c_int),
+                ("forced_step", C.c_int), ("traj_no", C.c_void_p), ("step_no", C.c_void_p), ("reset_count", C.c_void_p),
+                ("xy_off", C.c_void_p), ("qpos", C.c_void_p), ("qvel", C.c_void_p), ("obs_in", C.c_void_p),
+                ("obs", C.c_void_p), ("obs_dim", C.c_int), ("prev_x_vel", C.c_void_p), ("episode_step", C.c_void_p),
+                ("last", C.c_void_p), ("grf", C.c_void_p), ("n_grf", C.c_int), ("partial_resets", C.c_void_p),
+                ("model_index", C.c_void_p), ("mass", C.c_void_p), ("n_models", C.c_int), ("random", C.c_int),
+                ("masses_host", C.c_void_p)]
+
+
 class OmA3TaskDesc(C.Structure):
     _fields_ = [("period", C.c_int), ("delay_frames", C.c_int), ("target_radius", C.c_double),
                 ("goal_height_ref", C.c_double), ("goal_speed_ref", C.c_double), ("total_mass", C.c_double),
@@ -120,6 +130,7 @@ PROTOTYPES = {
                                       C.POINTER(OmPlayState), C.POINTER(OmPlayOut), _I, _I, _P]),
     "om_h1_live_step": (_I, [_P, C.POINTER(OmH1Spec), _P, _U64, _U32, C.POINTER(OmLiveState), C.POINTER(OmLiveOut), _I, _I, _P]),
     "om_h1_draw_models": (_I, [_U64, _U32, _U32, _I, _I, _P, _P, _P, _I, _P]),
+    "om_h1_reset_envs": (_I, [_P, C.POINTER(OmH1Spec), _P, _U64, _U32, C.POINTER(OmH1ResetArgs), _I, _I, _P]),
     "om_a3_task_create": (_I, [C.POINTER(OmA3TaskDesc), C.POINTER(_P)]),
     "om_a3_task_destroy": (None, [_P]),
     "om_a3_task_step": (_I, [_P, _P, _P, _P, _P, _I, C.POINTER(OmA3State), C.POINTER(OmA3Out), _I, _I, _P]),

@@ -164,6 +164,9 @@ OM_HD U4 om_draw(uint64_t seed, uint32_t env, uint32_t count, uint32_t stream) {
   return philox4x32_10(U4{env, count, stream, 0u}, (uint32_t)seed, (uint32_t)(seed >> 32));
 }
 OM_HD int to_int(uint32_t x, int n) { return (int)mulhi32(x, (uint32_t)n); }
+// Streams (third counter word) in use: 0 trajectory resets, 16..30 the A3 reset, 32 the MultiMuJoCo model switch of a whole
+// reset() (om_h1_draw_models), 33 the model an env draws at its own partial reset (om_h1_reset_envs), 48 expert minibatches.
+constexpr uint32_t STREAM_PARTIAL_MODEL_RESET = 33u;   // utils/philox.py
 OM_HD float to_unit(uint32_t x) { return (float)(x >> 8) * (1.0f / 16777216.0f); }
 
 }  // namespace om

@@ -366,13 +366,12 @@ OM_HD void play_start_reset(const PlayArgs& a, const OmPlayState& src, const OmP
   const uint32_t rc = src.reset_count[e];
   traj_draw(a.t, a.seed, a.env_id0 + env, rc, tr, st);
   float samp[H1Dims<V>::KPAD];
-  traj_load_row(a.t, tr, st, samp);
+  traj_reset_row(a.t, tr, st, samp);
   dst.traj_no[e] = tr;
   dst.step_no[e] = st;
   dst.reset_count[e] = rc + 1;
   dst.xy_off[e] = a.t.xy[((size_t)tr * a.t.T + st) * 2];
   dst.xy_off[ld + e] = a.t.xy[((size_t)tr * a.t.T + st) * 2 + 1];
-  samp[0] = 0.f; samp[1] = 0.f;                  // x - x_off and y - y_off are exactly zero at the reset sample
 #pragma unroll
   for (int k = 0; k < K; ++k) dst.pending[k * ld + e] = samp[k];
   if (dst.curr_qpos) {
@@ -641,19 +640,6 @@ __global__ void __launch_bounds__(BLOCK) h1_live_step_kernel(LiveArgs a) {
 }  // namespace om
 
 using namespace om;
-
-struct OmTraj {
-  TrajDev d;
-  // Scratch of the time-parallel playback kernel (episode-start snapshot of the carried state), grown on demand
-  // and kept: a stream-ordered allocation per call cost more than the kernel whenever the pool had been trimmed.
-  // One playback call per handle may be in flight at a time.
-  mutable char* scratch = nullptr;
-  mutable size_t scratch_bytes = 0;
-  // fork / join of the observation-moments kernel beside the time-parallel playback kernel (both only READ the snapshot)
-  mutable cudaStream_t side = nullptr;
-  mutable cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-};
-
 
 #ifndef OM_H1_VARIANT
 extern "C" int om_traj_create(const double* table, int K, int n_traj, int T, OmTraj** out) {

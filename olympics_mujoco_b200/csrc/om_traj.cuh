@@ -34,6 +34,14 @@ OM_HD void traj_load_row(const TrajDev& t, int traj_no, int step_no, float (&sam
   }
 }
 
+// the sample a reset starts from: row (traj_no, step_no) with root x, y re-centred on that row (reset_trajectory,
+// trajectory.py:316-320) -- x - x_off and y - y_off are exactly zero there
+template <int KPAD>
+OM_HD void traj_reset_row(const TrajDev& t, int traj_no, int step_no, float (&samp)[KPAD]) {
+  traj_load_row(t, traj_no, step_no, samp);
+  samp[0] = 0.f; samp[1] = 0.f;
+}
+
 // get_current_sample (trajectory.py:381-387) for one env into a [K][ld] SoA array
 OM_HD void traj_write_sample(const TrajDev& t, int traj_no, int step_no, double ox, double oy, float* sample, int ld, int env) {
   const size_t row = (size_t)traj_no * t.T + step_no;
@@ -44,3 +52,16 @@ OM_HD void traj_write_sample(const TrajDev& t, int traj_no, int step_no, double 
 }
 
 }  // namespace om
+
+// the OmTraj handle of the C ABI (om_traj.cu creates it; om_reset.cu reads its table)
+struct OmTraj {
+  om::TrajDev d;
+  // Scratch of the time-parallel playback kernel (episode-start snapshot of the carried state), grown on demand
+  // and kept: a stream-ordered allocation per call cost more than the kernel whenever the pool had been trimmed.
+  // One playback call per handle may be in flight at a time.
+  mutable char* scratch = nullptr;
+  mutable size_t scratch_bytes = 0;
+  // fork / join of the observation-moments kernel beside the time-parallel playback kernel (both only READ the snapshot)
+  mutable cudaStream_t side = nullptr;
+  mutable cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+};

@@ -112,6 +112,8 @@ class UnitreeH1(BaseHumanoidRobot):
                                      use_absorbing_states=kwargs.get("use_absorbing_states", True))
         self._fused_reward = hasattr(rf, "_target_vel")
         self._prev_x_vel = torch.zeros(self.n_envs, device=self._device)
+        # steps since each env's last reset (mushroom Core's episode_steps); advanced by step(autoreset=True)
+        self.episode_step = torch.zeros(self.n_envs, dtype=torch.int32, device=self._device)
 
     # ------------------------------------------------------------------ per-env carried weight
     def _bind_env_weights(self):
@@ -123,6 +125,8 @@ class UnitreeH1(BaseHumanoidRobot):
         self._weight_masses = [float(m.body_mass[self._weight_body]) for m in self._models]
         self.model_index = torch.zeros(self.n_envs, dtype=torch.int32, device=self._device)
         self.weight_body_mass = torch.full((self.n_envs,), self._weight_masses[0], dtype=torch.float32, device=self._device)
+        # each env's number of partial resets (reset(mask=...), step(autoreset=True)): the counter of its own model draw
+        self.partial_resets = torch.zeros(self.n_envs, dtype=torch.int32, device=self._device)
         Kn.bind_env_body_mass(self._dm, self._weight_body, self.weight_body_mass)
 
     def _draw_env_models(self, count):
@@ -200,11 +204,66 @@ class UnitreeH1(BaseHumanoidRobot):
                                           **kwargs)
 
     # ------------------------------------------------------------------ step (mushroom MuJoCo.step, SURVEY.md A.2)
-    def reset(self, obs=None):
-        out = super().reset(obs)
-        self._prev_x_vel.copy_(self._obs[:, self._spec.x_vel_idx])
+    def reset(self, obs=None, mask=None):
+        """``mask=None``: reset every env (loco_env_base.py:568-604).  ``mask`` ([n] bool or uint8 tensor on the env's
+        device): reset only the envs it selects, each exactly as reset() resets it, in one kernel (``om_h1_reset_envs``)
+        and without a host synchronisation -- qpos = qpos0 and qvel = 0, the GRF row zeroed (use_foot_forces), the
+        trajectory reset under the random_start / init_step_no rules of setup() (the om_traj_reset draw contract;
+        reset_count += 1), set_sim_state of its sample, the observation of that state, prev_x_vel and episode_step = 0.
+        Every state tensor of the other envs stays as it was; the FK mirrors (data.xpos, ...) are not written, as reset()
+        leaves them.  Returns the full [n, D] observation: the new rows of the reset envs, the current ones of the others.
+
+        Model switch of a masked reset: with ``per_env_weight`` env e draws its own model at its own partial resets --
+        ``philox_randint(seed, env_id0 + e, j, 33, 4)`` with j = ``partial_resets[e]`` (then incremented), or
+        ``(model_index[e] + 1) mod 4`` in round robin; the full reset() keeps its own contract (stream 32, the object's
+        reset count).  With a shared MultiMuJoCo (a carried weight of every valid mass without ``per_env_weight``) all envs
+        hold the object's one model, so only a reset of the whole object switches it: a masked reset neither switches the
+        model nor advances the object's reset count.  ``mask`` together with ``obs`` raises ValueError."""
+        if mask is None:
+            out = super().reset(obs)
+            self._prev_x_vel.copy_(self._obs[:, self._spec.x_vel_idx])
+            self.episode_step.zero_()
+            self._play_state = None
+            return out
+        if obs is not None:
+            raise ValueError("reset(obs=..., mask=...) is not supported: a masked reset draws from the trajectory")
+        if not torch.is_tensor(mask) or mask.dtype not in (torch.bool, torch.uint8) or tuple(mask.shape) != (self.n_envs,) \
+                or mask.device.type != torch.device(self._device).type:
+            raise ValueError(f"mask must be a [{self.n_envs}] bool or uint8 tensor on the env's device")
+        cur = self._obs
+        if cur is None:                              # never reset: the other envs keep the observation of their state
+            cur = self._create_observation(self.obs_helper._build_obs(self._data))
+        obs_in = cur.t().contiguous()
+        new = torch.empty_like(obs_in)
+        self._reset_envs(mask=mask, obs_in=obs_in, obs=new)
+        self._obs = new.t()
         self._play_state = None
-        return out
+        return self._out(self._modify_observation(self._obs))
+
+    def _reset_envs(self, obs_in, obs, mask=None, absorbing=None):
+        """om_h1_reset_envs with this env's state: the envs of ``mask``, or (mask=None) the auto-reset after a step."""
+        if self.trajectories is None:
+            raise ValueError("a per-env reset draws from the trajectory: load one first")
+        if self._init_step_no is not None and self._random_start:
+            raise ValueError("Either use a random start or set an initial step, not both.")
+        forced_traj, forced_step = -1, -1                                # setup() :640-657
+        if not self._random_start:
+            if self._init_step_no:
+                traj_len = self.trajectories.trajectory_length
+                assert self._init_step_no <= traj_len * self.trajectories.number_of_trajectories
+                forced_traj, forced_step = int(self._init_step_no / traj_len), int(self._init_step_no % traj_len)
+            else:
+                forced_step = 0
+        d = self._data
+        draw = {}
+        if self._per_env_model:
+            draw = dict(partial_resets=self.partial_resets, model_index=self.model_index, mass=self.weight_body_mass,
+                        masses=self._weight_masses, random=self._random_env_reset)
+        last = None if mask is not None else torch.empty(self.n_envs, dtype=torch.uint8, device=self._device)
+        Kn.h1_reset_envs(self._dm, self._spec, self.trajectories.device_state, d.qpos, d.qvel, mask=mask, absorbing=absorbing,
+                         horizon=self.info.horizon, forced_traj=forced_traj, forced_step=forced_step, obs_in=obs_in, obs=obs,
+                         prev_x_vel=self._prev_x_vel, episode_step=self.episode_step, last=last, grf=self._grf, **draw)
+        return last
 
     def attach_dynamics(self, fn, soa=False):
         """``soa=True``: ``fn(env, ctrl [nu, n]) -> (qpos [nq, n], qvel [nv, n])`` float32 CUDA tensors in the kernels' own
@@ -220,9 +279,16 @@ class UnitreeH1(BaseHumanoidRobot):
             return res[0], res[1]
         return res
 
-    def step(self, action):
+    def step(self, action, autoreset=False):
         """action [n, nu] in [-1, 1] ([nu, n] with SoA dynamics) -> (obs, reward, absorbing, info).  The physics between
-        observations comes from the attached dynamics; everything after it is one fused kernel (K1 + K2)."""
+        observations comes from the attached dynamics; everything after it is one fused kernel (K1 + K2).
+
+        ``autoreset=True`` adds mushroom_rl Core's bookkeeping on the device, in one more kernel on the same stream and
+        without a host synchronisation: ``episode_step += 1``, ``last = absorbing | (episode_step >= info.horizon)``, and
+        every env with ``last`` set gets the masked reset of ``reset(mask=last)``.  ``obs`` is then the observation after
+        those resets (the input to the next action); ``reward`` and ``absorbing`` are the step's own; ``info["last"]`` ([n]
+        bool) and ``info["final_obs"]`` -- the step's own observation of EVERY env, the ``next_state`` of the transition
+        (with use_foot_forces it carries the step's GRF / 1000, the reset rows of ``obs`` zeros)."""
         if self._dynamics is None:
             raise RuntimeError("step() needs a dynamics backend: env.attach_dynamics(fn).  Contact dynamics "
                                "(mj_step) are outside this package's hot path.")
@@ -245,6 +311,8 @@ class UnitreeH1(BaseHumanoidRobot):
             d.qvel.copy_(torch.as_tensor(qvel, device=self._device, dtype=torch.float32).reshape(self.n_envs, -1).t())
             qpos, qvel = d.qpos, d.qvel
         prev_obs = self._obs
+        if autoreset:
+            return self._step_autoreset(prev_obs, ctrl, qpos, qvel)
         out = Kn.h1_step(self._dm, self._spec, qpos, qvel, self._prev_x_vel,
                          out=dict(xpos=d.xpos, xquat=d.xquat, site_xpos=d.site_xpos, cvel=d.cvel))
         cur_obs = out["obs"].t()
@@ -255,6 +323,27 @@ class UnitreeH1(BaseHumanoidRobot):
         self._obs = cur_obs
         self._prev_x_vel.copy_(out["obs"][self._spec.x_vel_idx])
         return self._out(self._modify_observation(cur_obs)), self._out(reward), self._out(absorbing), {}
+
+    def _step_autoreset(self, prev_obs, ctrl, qpos, qvel):
+        """step(autoreset=True) after the dynamics: the step kernel writes the step's observation (the transition's
+        final_obs, [D, n] SoA with the GRF rows appended), then om_h1_reset_envs in auto-reset mode writes the returned
+        observation, last, episode_step and prev_x_vel and resets the envs whose episode ended."""
+        d = self._data
+        nobs = 2 * self._spec.n_obs_q - 2
+        final = torch.empty((nobs + (0 if self._grf is None else self._grf.shape[0]), self.n_envs), device=self._device)
+        out = Kn.h1_step(self._dm, self._spec, qpos, qvel, self._prev_x_vel,
+                         out=dict(xpos=d.xpos, xquat=d.xquat, site_xpos=d.site_xpos, cvel=d.cvel, obs=final[:nobs]))
+        if self._grf is not None:                                  # _create_observation: append mean_grf / 1000
+            torch.div(self._grf, 1000.0, out=final[nobs:])
+        final_obs = final.t()
+        absorbing = out["absorbing"].view(torch.bool)                # 0 / 1 bytes: a view, no copy
+        reward = out["reward"] if self._fused_reward else self.reward(prev_obs, ctrl, final_obs, absorbing)
+        new = torch.empty_like(final)
+        last = self._reset_envs(obs_in=final, obs=new, absorbing=out["absorbing"])
+        self._obs = new.t()
+        self._play_state = None
+        info = dict(last=self._out(last.view(torch.bool)), final_obs=self._out(self._modify_observation(final_obs)))
+        return self._out(self._modify_observation(self._obs)), self._out(reward), self._out(absorbing), info
 
     # ------------------------------------------------------------------ fused live step / graph
     def _has_fused_kernels(self):

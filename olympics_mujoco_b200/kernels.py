@@ -12,7 +12,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (OmA3Out, OmA3Returns, OmA3State, OmA3TaskDesc, OmActionSpec, OmDiscDesc, OmH1Spec, OmLiveOut, OmLiveState, OmMirrorSpec,
+from ._lib import (OmA3Out, OmA3Returns, OmA3State, OmA3TaskDesc, OmActionSpec, OmDiscDesc, OmH1ResetArgs, OmH1Spec, OmLiveOut, OmLiveState, OmMirrorSpec,
                    OmPdSpec, OmModelDesc, OmPlayOut, OmPlayState, check)
 from .mjcf import KinematicModel
 
@@ -106,6 +106,38 @@ def h1_draw_models(seed, env_id0, count, body_masses, idx, mass, random=True):
     assert mass.numel() == n
     check(_lib.load().om_h1_draw_models(int(seed), int(env_id0), int(count), len(bm), int(bool(random)), bm.ctypes.data,
                                         _p(idx, torch.int32), _p(mass, torch.float32), n, _stream()))
+
+
+def h1_reset_envs(dm, spec, traj, qpos, qvel, mask=None, absorbing=None, horizon=0, forced_traj=-1, forced_step=-1,
+                  obs_in=None, obs=None, prev_x_vel=None, episode_step=None, last=None, grf=None, partial_resets=None,
+                  model_index=None, mass=None, masses=(), random=True, n=None):
+    """``om_h1_reset_envs``: LocoEnvBase.reset for the envs of ``mask`` ([ld] bool / uint8), or -- ``mask=None`` -- the
+    auto-reset after a step: ``episode_step += 1``, ``last = absorbing | (episode_step >= horizon)``, reset where ``last``.
+    Everything is updated in place on the current stream: the trajectory state of ``traj``, qpos [nq, ld], qvel [nv, ld],
+    obs [D, ld] (from ``obs_in`` for the envs that do not reset), prev_x_vel, episode_step, last [ld] uint8, grf [G, ld]
+    and -- per-env models -- partial_resets, model_index (int32), mass (float32) from the host list ``masses``.
+    ld = ``traj.n`` (the width of its state tensors); ``n`` (default ld) envs are processed."""
+    _lib.require_cuda()
+    ld = traj.n
+    n = ld if n is None else int(n)
+    for name, t in (("qpos", qpos), ("qvel", qvel), ("obs_in", obs_in), ("obs", obs), ("grf", grf)):
+        if t is not None and t.shape[-1] != ld:
+            raise ValueError(f"{name} must be a [C, {ld}] SoA tensor")
+    if mask is not None and (mask.dtype not in (torch.bool, torch.uint8) or mask.shape != (ld,)):
+        raise ValueError(f"mask must be a [{ld}] bool or uint8 tensor")
+    i32, f32, u8 = torch.int32, torch.float32, torch.uint8
+    bm = np.ascontiguousarray(masses, dtype=np.float64)
+    v = lambda t, dt_=None: None if t is None else _p(t, dt_).value
+    a = OmH1ResetArgs(mask=v(mask), absorbing=v(absorbing, u8), horizon=int(horizon), forced_traj=int(forced_traj),
+                      forced_step=int(forced_step), traj_no=v(traj.traj_no, i32), step_no=v(traj.step_no, i32),
+                      reset_count=v(traj.reset_count, i32), xy_off=v(traj.xy_off, torch.float64), qpos=v(qpos, f32),
+                      qvel=v(qvel, f32), obs_in=v(obs_in, f32), obs=v(obs, f32), obs_dim=0 if obs is None else obs.shape[0],
+                      prev_x_vel=v(prev_x_vel, f32), episode_step=v(episode_step, i32), last=v(last, u8), grf=v(grf, f32),
+                      n_grf=0 if grf is None else grf.shape[0], partial_resets=v(partial_resets, i32),
+                      model_index=v(model_index, i32), mass=v(mass, f32), n_models=len(bm), random=int(bool(random)),
+                      masses_host=bm.ctypes.data if len(bm) else None)
+    check(_lib.load().om_h1_reset_envs(dm.handle, C.byref(spec), traj.handle, traj.seed, traj.env_id0, C.byref(a), n, ld,
+                                       _stream()))
 
 
 def fk(dm: DeviceModel, qpos, qvel=None, want=("xpos", "xquat", "site_xpos", "site_xmat", "cvel", "subtree_com"),

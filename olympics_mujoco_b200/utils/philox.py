@@ -4,7 +4,8 @@ takes (which model a MultiMuJoCo reset switches to, loco_env_base.py:586-589).""
 
 _M0, _M1, _W0, _W1, _MASK = 0xD2511F53, 0xCD9E8D57, 0x9E3779B9, 0xBB67AE85, 0xFFFFFFFF
 
-STREAM_MODEL_RESET = 32
+STREAM_MODEL_RESET = 32            # the model switch of a whole reset() (MultiMuJoCo; om_h1_draw_models)
+STREAM_PARTIAL_MODEL_RESET = 33    # the model one env draws at its own partial reset (om_h1_reset_envs)
 
 
 def philox4x32_10(counter, key):
@@ -32,3 +33,13 @@ def env_model_draw(seed, env_id, count, n_models, random=True):
     if random:
         return philox_randint(seed, env_id, count, STREAM_MODEL_RESET, n_models)
     return (int(env_id) + int(count) + 1) % int(n_models)
+
+
+def env_partial_model_draw(seed, env_id, j, n_models, prev_index, random=True):
+    """The model env ``env_id`` (global id) holds after its own ``j``-th partial reset (0-based; ``reset(mask=...)`` or
+    ``step(autoreset=True)`` with ``per_env_weight``; ``om_h1_reset_envs`` on the device): random -- the draw of stream 33
+    keyed on the env and its partial-reset count; round robin -- the model after ``prev_index``.  A stream of its own, so the
+    draws of whole resets (stream 32, ``env_model_draw``) never meet these."""
+    if random:
+        return philox_randint(seed, env_id, j, STREAM_PARTIAL_MODEL_RESET, n_models)
+    return (int(prev_index) + 1) % int(n_models)
