@@ -331,6 +331,29 @@ int om_a3_task_rollout(const OmModel* m, const OmA3Task* task, const float* qpos
 int om_a3_reset(const OmModel* m, const OmA3Task* task, uint64_t seed, uint32_t env_id0, const uint8_t* mask,
                 uint32_t* reset_count, double iteration_count, float* qpos, float* qvel, const OmA3State* state,
                 float* obs, int n, int ld, void* stream);
+/* Auto-reset after a one-step om_a3_task_step: the path bookkeeping of the PPO sampler (rl/algos/ppo.py:150-198: a path
+ * runs until done or max_traj_len steps, then the worker resets its env).  For every env i:
+ *   traj_len[i] += 1;  trunc = max_traj_len > 0 && traj_len[i] >= max_traj_len;  last[i] = done[i] || trunc;
+ *   path_end[i] = 1 if done[i] (bootstrap 0; wins over a truncation on the same step), 2 if trunc (bootstrap V(obs_in
+ *   row i), the step's own observation), else 0 -- the codes om_ppo_returns reads;
+ *   if last[i]: the reset of om_a3_reset (same draw contract: counter (env_id0 + i, reset_count[i], 16 + block, 0), then
+ *   reset_count[i] += 1; step height from iteration_count) writes qpos, qvel, the task state and obs row i; traj_len[i] = 0;
+ *   otherwise obs row i = obs_in row i (obs_in may equal obs).
+ * Nothing of an env that does not reset is written except its obs row, traj_len, last and path_end.  obs_in / obs [41][ld];
+ * done, last, path_end [ld] uint8; traj_len [ld] int32.  Every pointer is required.  The call only enqueues one kernel (no
+ * allocation, no host synchronisation): capturable in a CUDA graph behind om_a3_task_step. */
+typedef struct OmA3AutoResetArgs {
+  const uint8_t* done;          /* [ld] the step's done flags (OmA3Out.done) */
+  int max_traj_len;             /* 0 = no limit: only done ends a path */
+  double iteration_count;       /* env.robot.iteration_count (reset step heights, walking_task.py:378) */
+  uint32_t* reset_count; int32_t* traj_len;
+  float* qpos; float* qvel;     /* [25][ld], [24][ld] */
+  OmA3State state;
+  const float* obs_in; float* obs;
+  uint8_t* last; uint8_t* path_end;
+} OmA3AutoResetArgs;
+int om_a3_autoreset(const OmModel* m, const OmA3Task* task, uint64_t seed, uint32_t env_id0, const OmA3AutoResetArgs* args,
+                    int n, int ld, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K4: discriminator reward  r = -log(1 - sigmoid(D(s)) + 1e-8)  (GAIL.make_discrim_reward,

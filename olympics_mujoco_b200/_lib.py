@@ -84,6 +84,13 @@ class OmA3Returns(C.Structure):
                 ("gamma", C.c_float), ("ret", C.c_void_p), ("adv", C.c_void_p)]
 
 
+class OmA3AutoResetArgs(C.Structure):
+    _fields_ = [("done", C.c_void_p), ("max_traj_len", C.c_int), ("iteration_count", C.c_double),
+                ("reset_count", C.c_void_p), ("traj_len", C.c_void_p), ("qpos", C.c_void_p), ("qvel", C.c_void_p),
+                ("state", OmA3State), ("obs_in", C.c_void_p), ("obs", C.c_void_p), ("last", C.c_void_p),
+                ("path_end", C.c_void_p)]
+
+
 class OmDiscDesc(C.Structure):
     _fields_ = [("kind", C.c_int), ("n_in", C.c_int), ("n_h1", C.c_int), ("n_h2", C.c_int), ("z_size", C.c_int)] + \
                [(k, C.c_void_p) for k in ("w1", "b1", "w2", "b2", "wmu", "bmu", "wlv", "blv", "wd", "bd")]
@@ -136,6 +143,7 @@ PROTOTYPES = {
     "om_a3_task_step": (_I, [_P, _P, _P, _P, _P, _I, C.POINTER(OmA3State), C.POINTER(OmA3Out), _I, _I, _P]),
     "om_a3_task_rollout": (_I, [_P, _P, _P, _P, _P, _I, C.POINTER(OmA3State), C.POINTER(OmA3Out), C.POINTER(OmA3Returns), _I, _I, _P]),
     "om_a3_reset": (_I, [_P, _P, _U64, _U32, _P, _P, _D, _P, _P, C.POINTER(OmA3State), _P, _I, _I, _P]),
+    "om_a3_autoreset": (_I, [_P, _P, _U64, _U32, C.POINTER(OmA3AutoResetArgs), _I, _I, _P]),
     "om_disc_create": (_I, [C.POINTER(OmDiscDesc), C.POINTER(_P)]),
     "om_disc_destroy": (None, [_P]),
     "om_disc_reward": (_I, [_P, _P, _P, _P, _P, _I, _I, _P, _P, _P]),

@@ -382,10 +382,11 @@ struct A3ResetArgs {
   int n, ld;
 };
 
-__global__ void __launch_bounds__(128) a3_reset_kernel(A3ResetArgs a) {
-  const int env = blockIdx.x * blockDim.x + threadIdx.x;
-  if (env >= a.n) return;
-  if (a.mask && !a.mask[env]) return;
+// The reset of one env: the draws of counter reset_count[env] (then incremented), pose, FK for the foot positions
+// transform_sequence reads, WalkingTask.reset; writes qpos, qvel, the task ints, the footstep plan and -- a.obs not NULL --
+// the first observation.  Shared by the masked reset and the auto-reset after a step (Args: A3ResetArgs, A3AutoResetArgs).
+template <class Args>
+__device__ __forceinline__ void a3_reset_env(const Args& a, int env) {
   const size_t ld = a.ld, e = env;
   const uint32_t rc = a.reset_count[e];
   a.reset_count[e] = rc + 1;
@@ -413,6 +414,54 @@ __global__ void __launch_bounds__(128) a3_reset_kernel(A3ResetArgs a) {
     for (int k = 33; k < A3_NOBS; ++k) obs[k] = 0.f;
 #pragma unroll
     for (int k = 0; k < A3_NOBS; ++k) a.obs[k * ld + e] = obs[k];
+  }
+}
+
+__global__ void __launch_bounds__(128) a3_reset_kernel(A3ResetArgs a) {
+  const int env = blockIdx.x * blockDim.x + threadIdx.x;
+  if (env >= a.n) return;
+  if (a.mask && !a.mask[env]) return;
+  a3_reset_env(a, env);
+}
+
+// The PPO sampler's path bookkeeping after one step (rl/algos/ppo.py:150-198): traj_len += 1; the path ends on done or at
+// max_traj_len (0 = never); path_end = 1 (done: bootstrap 0, wins over a truncation on the same step), 2 (truncated:
+// bootstrap V(final obs)) or 0; an env whose path ended is reset exactly as a3_reset_kernel resets it.  obs = the step's
+// observation (obs_in) where no reset happened, the new first observation where one did.
+struct A3AutoResetArgs {
+  A3TaskConst C;
+  const float* init_qpos;
+  uint64_t seed;
+  uint32_t env_id0;
+  float step_h;
+  int max_traj_len;
+  const uint8_t* done;
+  uint32_t* reset_count; int32_t* traj_len;
+  float* qpos; float* qvel; int32_t* ints; float* sequence;
+  const float* obs_in; float* obs;
+  uint8_t* last; uint8_t* path_end;
+  int n, ld;
+};
+
+__global__ void __launch_bounds__(128) a3_autoreset_kernel(A3AutoResetArgs a) {
+  const int env = blockIdx.x * blockDim.x + threadIdx.x;
+  if (env >= a.n) return;
+  const size_t ld = a.ld, e = env;
+  const bool done = a.done[e] != 0;
+  const int tl = a.traj_len[e] + 1;
+  const bool trunc = a.max_traj_len > 0 && tl >= a.max_traj_len;
+  const bool end = done || trunc;
+  a.last[e] = end ? 1 : 0;
+  a.path_end[e] = done ? 1 : (trunc ? 2 : 0);
+  a.traj_len[e] = end ? 0 : tl;
+  if (end) {
+    a3_reset_env(a, env);
+  } else if (a.obs != a.obs_in) {                                      // the step's observation stays the env's observation
+    float v[A3_NOBS];
+#pragma unroll
+    for (int k = 0; k < A3_NOBS; ++k) v[k] = a.obs_in[k * ld + e];
+#pragma unroll
+    for (int k = 0; k < A3_NOBS; ++k) a.obs[k * ld + e] = v[k];
   }
 }
 
@@ -571,6 +620,13 @@ extern "C" int om_a3_task_rollout(const OmModel* m, const OmA3Task* task, const 
   return a3_step_impl(m, task, qpos, qvel, contact, n_steps, state, out, returns, n, ld, stream);
 }
 
+// WalkingTask.reset's step height for the curriculum position iteration_count (walking_task.py:378)
+static float a3_step_height(double iteration_count) {
+  double h = (iteration_count - 3000.0) / 8000.0;
+  h = (h < 0.0 ? 0.0 : (h > 1.0 ? 1.0 : h)) * 0.1;
+  return (float)h;
+}
+
 extern "C" int om_a3_reset(const OmModel* m, const OmA3Task* task, uint64_t seed, uint32_t env_id0, const uint8_t* mask,
                            uint32_t* reset_count, double iteration_count, float* qpos, float* qvel, const OmA3State* state,
                            float* obs, int n, int ld, void* stream) {
@@ -579,11 +635,29 @@ extern "C" int om_a3_reset(const OmModel* m, const OmA3Task* task, uint64_t seed
   OM_REQUIRE(n >= 0 && ld >= n, "om_a3_reset: need 0 <= n <= ld");
   if (n == 0) return 0;
   OM_REQUIRE(reset_count && qpos && qvel && state->ints && state->sequence, "om_a3_reset: null state");
-  double h = (iteration_count - 3000.0) / 8000.0;                      // walking_task.py:378
-  h = (h < 0.0 ? 0.0 : (h > 1.0 ? 1.0 : h)) * 0.1;
-  A3ResetArgs a{task->C, task->init_qpos, seed, env_id0, mask, reset_count, (float)h, qpos, qvel, state->ints,
-                state->sequence, obs, n, ld};
+  A3ResetArgs a{task->C, task->init_qpos, seed, env_id0, mask, reset_count, a3_step_height(iteration_count), qpos, qvel,
+                state->ints, state->sequence, obs, n, ld};
   a3_reset_kernel<<<ceil_div(n, 128), 128, 0, (cudaStream_t)stream>>>(a);
+  OM_LAUNCHED();
+  return 0;
+}
+
+extern "C" int om_a3_autoreset(const OmModel* m, const OmA3Task* task, uint64_t seed, uint32_t env_id0,
+                               const OmA3AutoResetArgs* args, int n, int ld, void* stream) {
+  OM_REQUIRE(m && task && args, "om_a3_autoreset: null argument");
+  OM_REQUIRE(m->specialised == SPEC_A3, "om_a3_autoreset: model is not the StickFigureA3 model");
+  OM_REQUIRE(n >= 0 && ld >= n, "om_a3_autoreset: need 0 <= n <= ld (n=%d ld=%d)", n, ld);
+  const OmA3AutoResetArgs& r = *args;
+  OM_REQUIRE(r.max_traj_len >= 0, "om_a3_autoreset: max_traj_len %d < 0 (0 = no limit)", r.max_traj_len);
+  if (n == 0) return 0;
+  OM_REQUIRE(r.done && r.reset_count && r.traj_len && r.qpos && r.qvel && r.state.ints && r.state.sequence && r.obs_in &&
+             r.obs && r.last && r.path_end,
+             "om_a3_autoreset: null input / state (done, reset_count, traj_len, qpos, qvel, state, obs_in, obs, last and "
+             "path_end are required)");
+  A3AutoResetArgs a{task->C, task->init_qpos, seed, env_id0, a3_step_height(r.iteration_count), r.max_traj_len, r.done,
+                    r.reset_count, r.traj_len, r.qpos, r.qvel, r.state.ints, r.state.sequence, r.obs_in, r.obs, r.last,
+                    r.path_end, n, ld};
+  a3_autoreset_kernel<<<ceil_div(n, 128), 128, 0, (cudaStream_t)stream>>>(a);
   OM_LAUNCHED();
   return 0;
 }

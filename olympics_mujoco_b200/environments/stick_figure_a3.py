@@ -5,7 +5,11 @@
 ``step(a)`` keeps the reference's contract ``(obs, total_reward, done, rewards_dict)`` for n envs.  The physics
 between two observations (``robot.step`` -> frame_skip x [PD law -> ``mj_step``]) is NOT part of this path: it is an
 attached callable returning the post-physics ``qpos``, ``qvel`` and the four contact-solver summaries the task reads;
-everything after it runs in one fused CUDA kernel (``om_a3_task_step``)."""
+everything after it runs in one fused CUDA kernel (``om_a3_task_step``).
+
+``step(a, autoreset=True, max_traj_len=L)`` adds the path bookkeeping of the reference's PPO sampler
+(``rl/algos/ppo.py:150-198``) in one more kernel (``om_a3_autoreset``) on the same stream: each env counts the steps of its
+path (``traj_len``), a path ends on ``done`` or after ``L`` steps, and an env whose path ended is reset alone."""
 from __future__ import annotations
 
 import numpy as np
@@ -81,6 +85,8 @@ class StickFigureA3:
         self.qpos = Kn.soa(self._model.nq, self.n_envs, device=device)
         self.qvel = Kn.soa(self._model.nv, self.n_envs, device=device)
         self._obs = Kn.soa(41, self.n_envs, device=device)
+        # steps of each env's current path (the sampler's traj_len); advanced by step(autoreset=True)
+        self.traj_len = torch.zeros(self.n_envs, dtype=torch.int32, device=device)
         self._dynamics = None
 
     # ------------------------------------------------------------------ helpers
@@ -97,18 +103,34 @@ class StickFigureA3:
 
     # ------------------------------------------------------------------ reset / step
     def reset_model(self, mask=None):
-        """StickFigureA3.py:205-235 (+ WalkingTask.reset) for every env, or the envs selected by ``mask``."""
+        """StickFigureA3.py:205-235 (+ WalkingTask.reset) for every env, or the envs selected by ``mask``; their
+        ``traj_len`` restarts at 0."""
         if mask is not None:
             mask = torch.as_tensor(mask, device=self._device).to(torch.uint8)
         self._dev.reset(self.qpos, self.qvel, mask=mask, iteration_count=self.robot.iteration_count, obs=self._obs)
+        if mask is None:
+            self.traj_len.zero_()
+        else:
+            self.traj_len.masked_fill_(mask.bool(), 0)
         return self.get_obs()
 
     def reset(self, obs=None):
         """loco_env_base.py:577-579 -> test_reset :220-223 -> reset_model."""
         return self.reset_model()
 
-    def step(self, a):
-        """StickFigureA3.py:187-202."""
+    def step(self, a, autoreset=False, max_traj_len=None):
+        """StickFigureA3.py:187-202 -> (obs, reward, done, rewards dict).
+
+        ``autoreset=True`` runs the reference's PPO sampler loop (rl/algos/ppo.py:150-198) on the device, after the step
+        kernel and without a host synchronisation: ``traj_len += 1``; a path ends on ``done`` or when ``traj_len`` reaches
+        ``max_traj_len`` (None: only ``done`` ends it); every env whose path ended is reset exactly as
+        ``reset_model(mask=last)`` resets it.  ``obs`` is then the observation after those resets (the next action's
+        input); ``reward`` and ``done`` are the step's own.  The dict gains ``last`` ([n] bool), ``path_end`` ([n] uint8: 1
+        done -- bootstrap 0, it wins over a truncation on the same step; 2 truncated -- bootstrap V(final_obs); 0 the path
+        goes on: the codes of ``learners.finish_path``), ``final_obs`` ([n, 41], the step's observation of every env: the
+        ``next_state`` V is evaluated on at a truncation) and ``traj_len`` ([n] int32, after the update)."""
+        if max_traj_len is not None and int(max_traj_len) < 1:
+            raise ValueError(f"max_traj_len must be None or >= 1, got {max_traj_len}")
         if self._dynamics is None:
             raise RuntimeError("StickFigureA3.step needs the physics: call attach_dynamics(fn) first "
                                "(contact dynamics are outside this package)")
@@ -121,8 +143,26 @@ class StickFigureA3:
         self.qpos.copy_(qpos)
         self.qvel.copy_(qvel)
         self.robot.prev_action = target
+        if autoreset:
+            return self._step_autoreset(contact.contiguous(), max_traj_len)
         out = self._dev.step(self.qpos, self.qvel, contact.contiguous(), out=dict(obs=self._obs))
         rewards = {k: self._out(out["terms"][i]) for i, k in enumerate(REWARD_KEYS)}
+        return self.get_obs(), self._out(out["reward"]), self._out(out["done"].bool()), rewards
+
+    def _step_autoreset(self, contact, max_traj_len):
+        """step(autoreset=True) after the physics: the step kernel writes the step's observation (final_obs), then
+        om_a3_autoreset writes the returned observation, traj_len, last and path_end and resets the envs whose path ended."""
+        final = Kn.soa(41, self.n_envs, device=self._device)
+        out = self._dev.step(self.qpos, self.qvel, contact, out=dict(obs=final))
+        new = torch.empty_like(final)
+        last = torch.empty(self.n_envs, dtype=torch.uint8, device=self._device)
+        path_end = torch.empty_like(last)
+        self._dev.autoreset(self.qpos, self.qvel, out["done"], self.traj_len, final, new, last, path_end,
+                            max_traj_len=max_traj_len, iteration_count=self.robot.iteration_count)
+        self._obs = new
+        rewards = {k: self._out(out["terms"][i]) for i, k in enumerate(REWARD_KEYS)}
+        rewards.update(last=self._out(last.view(torch.bool)), path_end=self._out(path_end), final_obs=self._out(final.t()),
+                       traj_len=self._out(self.traj_len.clone()))
         return self.get_obs(), self._out(out["reward"]), self._out(out["done"].bool()), rewards
 
     def _has_fallen(self, obs, return_err_msg=False):

@@ -12,7 +12,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (OmA3Out, OmA3Returns, OmA3State, OmA3TaskDesc, OmActionSpec, OmDiscDesc, OmH1ResetArgs, OmH1Spec, OmLiveOut, OmLiveState, OmMirrorSpec,
+from ._lib import (OmA3AutoResetArgs, OmA3Out, OmA3Returns, OmA3State, OmA3TaskDesc, OmActionSpec, OmDiscDesc, OmH1ResetArgs, OmH1Spec, OmLiveOut, OmLiveState, OmMirrorSpec,
                    OmPdSpec, OmModelDesc, OmPlayOut, OmPlayState, check)
 from .mjcf import KinematicModel
 
@@ -400,6 +400,37 @@ class A3Task:
                                       _p(qvel, torch.float32), C.byref(st), _p(obs, torch.float32), self.n, max(self.n, 1),
                                       _stream()))
         return obs
+
+    def autoreset(self, qpos, qvel, done, traj_len, obs_in, obs, last, path_end, max_traj_len=None, iteration_count=0.0,
+                  n=None):
+        """``om_a3_autoreset``: the PPO sampler's path bookkeeping after a one-step ``step`` (rl/algos/ppo.py:150-198):
+        ``traj_len += 1``; a path ends on ``done`` or at ``max_traj_len`` (None = never); ``last`` = it ended, ``path_end`` =
+        1 (done) / 2 (truncated) / 0, the codes of ``ppo_returns``; an env whose path ended is reset as ``reset(mask=last)``
+        resets it and ``traj_len`` restarts at 0.  ``obs`` = ``obs_in`` (the step's observation) where no reset happened, the
+        new first observation where one did.  Everything in place on the current stream: qpos [25, ld], qvel [24, ld], the
+        task state, reset_count, traj_len (int32 [ld]), obs [41, ld], last / path_end ([ld] uint8 or bool).  done ([ld]
+        uint8 or bool), obs_in [41, ld].  ld = ``self.n``; ``n`` (default ld) envs are processed."""
+        ld = self.n
+        n = ld if n is None else int(n)
+        if not 0 <= n <= ld:
+            raise ValueError(f"n = {n} outside [0, {ld}]")
+        if max_traj_len is not None and int(max_traj_len) < 1:
+            raise ValueError(f"max_traj_len must be None or >= 1, got {max_traj_len}")
+        for name, t, rows in (("qpos", qpos, 25), ("qvel", qvel, 24), ("obs_in", obs_in, A3_NOBS), ("obs", obs, A3_NOBS)):
+            if t.shape != (rows, ld) or t.dtype != torch.float32:
+                raise ValueError(f"{name} must be a float32 [{rows}, {ld}] SoA tensor")
+        for name, t, dts in (("done", done, (torch.uint8, torch.bool)), ("last", last, (torch.uint8, torch.bool)),
+                             ("path_end", path_end, (torch.uint8,)), ("traj_len", traj_len, (torch.int32,))):
+            if t.shape != (ld,) or t.dtype not in dts:
+                raise ValueError(f"{name} must be a [{ld}] {' or '.join(str(d) for d in dts)} tensor")
+        _lib.require_cuda()
+        v = lambda t: _p(t).value
+        a = OmA3AutoResetArgs(done=v(done), max_traj_len=0 if max_traj_len is None else int(max_traj_len),
+                              iteration_count=float(iteration_count), reset_count=v(self.reset_count), traj_len=v(traj_len),
+                              qpos=v(qpos), qvel=v(qvel), state=self._state(), obs_in=v(obs_in), obs=v(obs), last=v(last),
+                              path_end=v(path_end))
+        check(_lib.load().om_a3_autoreset(self.dm.handle, self.handle, self.seed, self.env_id0, C.byref(a), n, max(ld, 1),
+                                          _stream()))
 
     def step(self, qpos, qvel, contact, want=("obs", "terms", "reward", "done"), out=None, returns=None):
         """The StickFigureA3.step tail on post-physics states.  qpos [25,n] (one step) or [T,25,n] (replay of T

@@ -34,7 +34,15 @@ def compute_gae(v, v_next, r, absorbing, last, gamma, lam, normalize=False):
 
 
 def finish_path(rewards, values, gamma, path_end=None, v_next=None, last_val=None):
-    """-> (returns, advantages = returns - values) for a rollout buffer; ``last_val`` = (not done) * V(s_T)."""
+    """-> (returns, advantages = returns - values) for a rollout buffer; ``last_val`` = (not done) * V(s_T).
+
+    Over a [T, n] buffer filled by ``StickFigureA3.step(a, autoreset=True, max_traj_len=L)``, with ``info["path_end"]``
+    and ``info["final_obs"]`` of every step stacked and ``obs_T`` the observation returned by the last step::
+
+        finish_path(rewards, values, gamma, path_end=path_end, v_next=V(final_obs), last_val=V(obs_T))
+
+    A path that ended by ``done`` bootstraps 0, one cut at ``max_traj_len`` bootstraps V of its own last observation, and
+    one still running at the end of the buffer bootstraps V(obs_T) -- the reference sampler's ``(not done) * V(state)``."""
     return Kn.ppo_returns(rewards, values, gamma, path_end=path_end, v_next=v_next, v_last=last_val)
 
 
